@@ -27,6 +27,13 @@ only collective).  Prints ONE JSON line (rank 0).
 `--impl reference` times only that CPU path on the same config (the reference is pure Python over torch/torchvision
 and does not exist on the GPU box; its algorithm is restated in oracle/ and pinned against the real reference by
 oracle/make_golden.py).
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as float32 .npy files, so that two
+builds can be compared output for output (inputs and weights are seeded, identical from run to run):
+  tokens       [images, 1+T] token ids (column 0 = sos, pad past the step count; N > 1: all ranks' images)
+  steps        decode steps executed (N > 1: one per rank)
+  score        beam search only: the best hypothesis' score of each of rank 0's images
+  tokens_rows  only when tokens alone would pass 64 MB: the fixed, seeded sample of rows kept in tokens
 """
 from __future__ import annotations
 
@@ -63,6 +70,7 @@ ENC_GFLOP = {"swin": 6.515, "res18": 2.24}       # reference-executed per image 
 ENC_GFLOP_MINIMAL = {"swin": 5.498, "res18": 2.24}
 MEM_TOKENS = {"swin": 30, "res18": 10}
 DEC_WEIGHT_PARAMS = 7_630_547
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -115,6 +123,26 @@ def decode_traffic_from_ncu(batch: int, T: int, beam: int):
     if sha is None or sha != kernel_source_sha():
         return None, "stale: profiles/decode_traffic.json (%s) was captured with other decode-kernel sources" % d.get("source")
     return d["dram_bytes_per_step"], "profiles/decode_traffic.json (%s, ncu capture of this kernel source, sha256 %s)" % (d.get("source"), sha[:12])
+
+
+def dump_outputs(out_dir: str, tokens, steps, score=None):
+    """Write the outputs of one step as DIR/<name>.npy (float32: token ids and step counts are exact), at most
+    DUMP_LIMIT_BYTES in all; past that, `tokens` keeps a fixed, seeded sample of its rows, listed in tokens_rows.npy."""
+    import numpy as np
+    arrays = {"steps": steps.cpu().numpy().astype(np.float32)}
+    if score is not None:
+        arrays["score"] = score.cpu().numpy().astype(np.float32)
+    tok = tokens.cpu().numpy().astype(np.float32)
+    budget = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values()) - 4 * 4096       # 4096: room for .npy headers
+    if tok.nbytes > budget:
+        keep = budget // (tok[0].nbytes + 4)
+        rows = np.sort(np.random.default_rng(0).choice(tok.shape[0], keep, replace=False))
+        arrays["tokens_rows"] = rows.astype(np.float32)
+        tok = tok[rows]
+    arrays["tokens"] = tok
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -207,7 +235,7 @@ def cpu_reference_sample(config: int, reps: int, warmup: int):
                 times.append(dt)
     steps = ys.shape[1] - 1
     return {"times": times, "images": n_images, "tokens": n_images * steps, "cores": torch.get_num_threads(),
-            "sample": f"{n_images} images x {max_len} steps in one batch per repetition, {what}"}
+            "sample": f"{n_images} images x {max_len} steps in one batch per repetition, {what}", "ys": ys}
 
 
 def cpu_b1_latency(reps: int = 2):
@@ -247,6 +275,9 @@ def run_reference(args, rank):
         "e2e": {"value": ips, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        ys = r["ys"]
+        dump_outputs(args.dump_outputs, ys, torch.tensor([ys.shape[1] - 1]))
     print(json.dumps(line), flush=True)
 
 
@@ -303,10 +334,14 @@ def run_ours(args, rank, local_rank, world):
         out = model.generate_device(x, max_len=T, beam_size=beam)
         return out[0], out[1]
 
+    last = {}      # device outputs of the latest step_device() call, for --dump-outputs
+
     def step_device():
-        tok, st = decode(dev_imgs)
+        out = model.generate_device(dev_imgs, max_len=T, beam_size=beam)
+        tok, st = out[0], out[1]
         if world > 1:      # stream-ordered: decode -> the path's only collective (NCCL all-gather of the ids)
             tok, st = gather_tokens_device(tok, st)
+        last.update(tokens=tok, steps=st, score=out[3] if beam > 1 else None)
         return tok, int(st.max().item())       # one host read per step
 
     def barrier():
@@ -333,6 +368,7 @@ def run_ours(args, rank, local_rank, world):
         enc_ms.append(e_ms); dec_ms.append(d_ms)
     barrier()
     wall = time.perf_counter() - wall0
+    timed_outputs = dict(last)
     launches = lib.hmocr_launch_count() - launches0
     clocks = sampler.stop()
     step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -487,6 +523,8 @@ def run_ours(args, rank, local_rank, world):
                 line["cpu_baseline"]["b1_p50_ms"] = cpu_b1_latency()
                 line["cpu_baseline"]["b1_sample"] = ("one image, 150 greedy steps, oracle port of src/predict.py:49-67 "
                                                      "(BASELINE.json configs[0]), median of 2")
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, **timed_outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -503,7 +541,11 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="override the config's images per GPU")
     ap.add_argument("--max-len", type=int, default=0, help="override the config's decode length")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
