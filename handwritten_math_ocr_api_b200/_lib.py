@@ -38,6 +38,7 @@ SIGNATURES = {
     "hmocr_decoder_forward": (_i, [_p, _p, _p, _i, _i, _p, _p]),
     "hmocr_generate": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_generate_from_memory": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
+    "hmocr_generate_nbest": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_generate_host": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_preprocess_u8": (_i, [_p, _p, _i, _p, _p]),
     "hmocr_pack_tokens": (_i, [_p, _p, _i, _i, _p, _p, _p]),

@@ -59,8 +59,8 @@ constexpr float LN_EPS = 1e-5f;
 struct __align__(16) Partial { float m; int idx; float s; int pad; };
 // beam search: K best (logit, token) of a row, best first; 48 bytes = three 16-byte DSMEM stores
 struct __align__(16) TopList { float v[DP_MAX_BEAM]; int i[DP_MAX_BEAM]; int pad[2]; };
-struct Cand { float score; int flat; };
-struct Sel { float score; int parent; int tok; };
+struct Cand { float score; int flat; float lp; };           // lp = log_softmax of the candidate's token
+struct Sel { float score; int parent; int tok; float lp; };
 
 struct Smem {
   alignas(128) uint8_t slot[NW][DP_CHUNK];  // warp-private weight slots
@@ -78,8 +78,8 @@ struct Smem {
   // beam search only
   TopList wtop[NW][R];                      // per-warp top-K logits of every row
   TopList ctop[CL][R];                      // per-CTA top-K, gathered from the 8 CTAs
-  Cand cand[R][DP_MAX_BEAM];                // candidate (score, hypothesis * V + token) of every row
-  Sel sel[R];                               // chosen (score, parent row, token) of every new hypothesis
+  Cand cand[R][DP_MAX_BEAM];                // candidate (score, hypothesis * V + token, log-prob) of every row
+  Sel sel[R];                               // chosen (score, parent row, token, log-prob) of every new hypothesis
   float bscore[R];
   int bfin[R], bsrc[R];
   alignas(8) uint64_t full[NW];
@@ -986,10 +986,10 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
 #pragma unroll
         for (int k = 0; k < KB; ++k) {
           Cand cd;
-          cd.score = -INFINITY; cd.flat = 0x7fffffff;
+          cd.score = -INFINITY; cd.flat = 0x7fffffff; cd.lp = 0.f;
           if (row_ok && k < p.beam) {
             if (fin) { if (k == 0) { cd.score = sc; cd.flat = hyp * p.vocab + p.pad; } }     // frozen: one candidate
-            else { cd.score = sc + (tl.v[k] - lse); cd.flat = hyp * p.vocab + tl.i[k]; }
+            else { cd.lp = tl.v[k] - lse; cd.score = sc + cd.lp; cd.flat = hyp * p.vocab + tl.i[k]; }
           }
           s.cand[warp][k] = cd;
         }
@@ -998,22 +998,24 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
       if (warp * p.beam < nrows) {           // warp i = image i of this cluster: K rounds of arg-best over K x KB candidates
         const int hyp = lane / KB, k = lane - hyp * KB;
         Cand cd;
-        cd.score = -INFINITY; cd.flat = 0x7fffffff;
+        cd.score = -INFINITY; cd.flat = 0x7fffffff; cd.lp = 0.f;
         if (hyp < p.beam) cd = s.cand[warp * p.beam + hyp][k];
         for (int j = 0; j < p.beam; ++j) {
-          float bv = cd.score;
+          float bv = cd.score, bl = cd.lp;
           int bf = cd.flat;
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) {
             const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
             const int of = __shfl_xor_sync(0xffffffffu, bf, o);
-            if (cand_before(ov, of, bv, bf)) { bv = ov; bf = of; }
+            const float ol = __shfl_xor_sync(0xffffffffu, bl, o);
+            if (cand_before(ov, of, bv, bf)) { bv = ov; bf = of; bl = ol; }
           }
           if (lane == 0) {
             Sel se;
             se.score = bv;
             se.parent = (bf == 0x7fffffff) ? warp * p.beam : warp * p.beam + bf / p.vocab;
             se.tok = (bf == 0x7fffffff) ? p.pad : bf % p.vocab;
+            se.lp = (bf == 0x7fffffff) ? 0.f : bl;
             s.sel[warp * p.beam + j] = se;
           }
           if (cd.flat == bf) { cd.score = -INFINITY; cd.flat = 0x7fffffff; }      // taken
@@ -1031,6 +1033,7 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
         if (c == 0) {
           p.bp_parent[(size_t)t * p.rows + row0 + warp] = me.parent % p.beam;     // clusters hold whole images
           p.bp_token[(size_t)t * p.rows + row0 + warp] = tok;
+          if (p.bp_logp != nullptr) p.bp_logp[(size_t)t * p.rows + row0 + warp] = me.lp;
           p.bm_tok[row0 + warp] = tok;
         }
       }
@@ -1120,25 +1123,36 @@ __global__ void beam_init_kernel(DecodeState* state, float* bm_score, int* bm_fi
   }
 }
 
+// One thread per hypothesis: its rank among the image's K hypotheses (score descending, ties -> lower beam index, so
+// rank 0 is the first maximum); ranks below n_best are back-tracked into slot [img][rank].
 __global__ void beam_finalize_kernel(const DecodeState* state, const float* bm_score, const int* bp_parent,
-                                     const int* bp_token, int images, int beam, int rows, int max_len, int sos, int pad,
-                                     int64_t* tokens, int ld_tok, float* score_out, int32_t* steps_out) {
+                                     const int* bp_token, const float* bp_logp, int images, int beam, int n_best,
+                                     int rows, int max_len, int sos, int pad, int64_t* tokens, float* logprob,
+                                     float* score_out, int32_t* steps_out) {
   const int steps = state->steps_executed > 0 ? state->steps_executed : min(state->step, max_len);
-  const int img = blockIdx.x * blockDim.x + threadIdx.x;
-  if (img == 0 && steps_out != nullptr) *steps_out = steps;
-  if (img >= images) return;
-  int best = 0;
-  float bs = bm_score[img * beam];
-  for (int j = 1; j < beam; ++j)
-    if (bm_score[img * beam + j] > bs) { bs = bm_score[img * beam + j]; best = j; }       // first max
-  if (score_out != nullptr) score_out[img] = bs;
-  int64_t* out = tokens + (size_t)img * ld_tok;
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r == 0 && steps_out != nullptr) *steps_out = steps;
+  if (r >= images * beam) return;
+  const int img = r / beam, j = r - img * beam;
+  const float* sc = bm_score + (size_t)img * beam;
+  auto key = [](float v) { return isnan(v) ? -INFINITY : v; };     // a strict total order: ranks are a permutation
+  const float mine = key(sc[j]);
+  int rank = 0;
+  for (int i = 0; i < beam; ++i) rank += key(sc[i]) > mine || (key(sc[i]) == mine && i < j);
+  if (rank >= n_best) return;
+  const size_t slot = (size_t)img * n_best + rank;
+  if (score_out != nullptr) score_out[slot] = sc[j];
+  int64_t* out = tokens + slot * (max_len + 1);
+  float* lp = logprob != nullptr ? logprob + slot * max_len : nullptr;
   out[0] = sos;
-  for (int k = steps + 1; k < ld_tok; ++k) out[k] = pad;
-  int b = best;
-  for (int t = steps - 1; t >= 0; --t) {
+  for (int k = steps + 1; k <= max_len; ++k) out[k] = pad;
+  if (lp != nullptr)
+    for (int k = steps; k < max_len; ++k) lp[k] = 0.f;
+  int b = j;
+  for (int t = steps - 1; t >= 0; --t) {     // a frozen hypothesis recorded (itself, pad, 0) after its eos
     const size_t at = (size_t)t * rows + img * beam + b;
     out[t + 1] = bp_token[at];
+    if (lp != nullptr) lp[t] = bp_logp[at];
     b = bp_parent[at];
   }
 }
@@ -1223,10 +1237,13 @@ int beam_init(cudaStream_t st, DecodeState* state, float* bm_score, int* bm_fin,
 }
 
 int beam_finalize(cudaStream_t st, const DecodeState* state, const float* bm_score, const int* bp_parent,
-                  const int* bp_token, int images, int beam, int rows, int max_len, int sos, int pad, int64_t* tokens,
-                  int ld_tok, float* score_out, int32_t* steps_out) {
-  beam_finalize_kernel<<<ceil_div(images, 128), 128, 0, st>>>(state, bm_score, bp_parent, bp_token, images, beam, rows,
-                                                              max_len, sos, pad, tokens, ld_tok, score_out, steps_out);
+                  const int* bp_token, const float* bp_logp, int images, int beam, int n_best, int rows, int max_len,
+                  int sos, int pad, int64_t* tokens, float* logprob, float* score_out, int32_t* steps_out) {
+  HM_CHECK(n_best >= 1 && n_best <= beam, "n_best=%d outside [1, beam=%d]", n_best, beam);
+  HM_CHECK(logprob == nullptr || bp_logp != nullptr, "beam_finalize: per-token log-probs were not recorded");
+  beam_finalize_kernel<<<ceil_div(images * beam, 128), 128, 0, st>>>(state, bm_score, bp_parent, bp_token, bp_logp, images,
+                                                                     beam, n_best, rows, max_len, sos, pad, tokens,
+                                                                     logprob, score_out, steps_out);
   HM_LAUNCHED();
   return 0;
 }

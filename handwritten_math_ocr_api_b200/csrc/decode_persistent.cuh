@@ -59,6 +59,7 @@ struct DecPersistParams {
   int* bm_tok;                // [rows] token fed at the next step
   int* bp_parent;             // [max_len][rows] beam index (within the image) of the parent chosen at step t
   int* bp_token;              // [max_len][rows] token chosen at step t
+  float* bp_logp;             // [max_len][rows] log-probability of that token (0 once frozen), or nullptr
   int num_layers, fc_tiles, chunks_per_step, vocab;
   int tmax, max_pos, max_len, ld_tok, eos, pad;
   long long* trace;           // optional: clock64() of cluster 0 / CTA 0 / thread 0 at every phase boundary
@@ -75,9 +76,11 @@ constexpr int DP_MAX_BEAM = 5;
 // beam search bookkeeping around the persistent kernel
 int beam_init(cudaStream_t st, DecodeState* state, float* bm_score, int* bm_fin, int* bm_src, int* bm_tok, int rows,
               int beam, int rows_per_cluster, int sos);
-// best hypothesis per image (highest score, ties -> lowest beam index), back-tracked through bp_parent / bp_token
+// n_best best hypotheses per image (score descending, ties -> lower beam index), back-tracked through bp_parent /
+// bp_token: tokens [images][n_best][1+max_len] (column 0 sos, pad past the steps executed), score_out [images][n_best],
+// logprob [images][n_best][max_len] from bp_logp (0 past the steps executed).  score_out, logprob, steps_out may be null.
 int beam_finalize(cudaStream_t st, const DecodeState* state, const float* bm_score, const int* bp_parent,
-                  const int* bp_token, int images, int beam, int rows, int max_len, int sos, int pad, int64_t* tokens,
-                  int ld_tok, float* score_out, int32_t* steps_out);
+                  const int* bp_token, const float* bp_logp, int images, int beam, int n_best, int rows, int max_len,
+                  int sos, int pad, int64_t* tokens, float* logprob, float* score_out, int32_t* steps_out);
 
 }  // namespace hmocr

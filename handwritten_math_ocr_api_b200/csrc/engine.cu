@@ -630,14 +630,19 @@ int enqueue_step(hmocr_engine* e, const GenBufs& g, int rows, const h16* memkv, 
 }
 
 int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam, int64_t* tokens,
-                        float* logprob, int32_t* steps, float* score, cudaStream_t st);
+                        float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best);
 
+// n_best == 0: the hmocr_generate contract (best hypothesis only; logprob zero-filled in beam mode).
+// n_best >= 1: the hmocr_generate_nbest contract (beam machinery always; tokens / logprob / score hold n_best
+// hypotheses per image).  The step-graph decode is greedy only, so n-best always takes the persistent kernel.
 int generate_from_memory_impl(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam,
-                              int64_t* tokens, float* logprob, int32_t* steps, float* score, cudaStream_t st) {
+                              int64_t* tokens, float* logprob, int32_t* steps, float* score, cudaStream_t st,
+                              int n_best = 0) {
   HM_CHECK(max_len >= 1 && max_len <= e->cfg.max_seq_len,
            "max_len=%d outside [1, %d] (size of pos_encoder, src/model_swin.py:54)", max_len, e->cfg.max_seq_len);
   HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
-  if (e->decode_impl == 0) return generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st);
+  if (e->decode_impl == 0 || n_best > 0)
+    return generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
   HM_CHECK(beam == 1, "the step-graph decode (decode_impl=1) is greedy only; beam=%d needs decode_impl=0", beam);
   const int d = e->cfg.d_model, nh = e->cfg.nhead, L = e->cfg.num_layers;
   const int rows = B;
@@ -795,9 +800,9 @@ int pack_decode_operands(hmocr_engine* e) {
 // (src/inference.py:15-25).  beam > 1 (or option "force_beam_kernel"): beam search as defined in
 // oracle/decode.py::beam_search - rows = images x beam hypotheses, two K/V cache sets, back-track at the end.
 int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam, int64_t* tokens,
-                        float* logprob, int32_t* steps, float* score, cudaStream_t st) {
+                        float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best) {
   const int nh = e->cfg.nhead, L = e->cfg.num_layers, rows = B * beam;
-  const bool beam_mode = beam > 1 || e->force_beam_kernel;
+  const bool beam_mode = beam > 1 || e->force_beam_kernel || n_best > 0;
   HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
   float* memkv;                       // memory K/V of all layers, fp32 out of the GEMM, fp16 after the repack
   __half *memk, *memv, *kcache, *vcache;
@@ -829,6 +834,7 @@ int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, i
     HM_TRY(ws_get(e, "bm.tok", rows, &p.bm_tok));
     HM_TRY(ws_get(e, "bm.parent", (size_t)max_len * rows, &p.bp_parent));
     HM_TRY(ws_get(e, "bm.token", (size_t)max_len * rows, &p.bp_token));
+    if (n_best > 0) HM_TRY(ws_get(e, "bm.logp", (size_t)max_len * rows, &p.bp_logp));
   }
   if (e->trace_step >= 0) HM_TRY(ws_get(e, "gen.trace", 1024, &p.trace));
   if (e->planning) return 0;
@@ -894,9 +900,12 @@ int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, i
       if (e->pinned_state[prev].steps_executed > 0) done = true;
     }
   }
-  if (beam_mode) {
-    HM_TRY(beam_finalize(st, state, p.bm_score, p.bp_parent, p.bp_token, B, beam, rows, max_len, e->cfg.sos_id,
-                         e->cfg.pad_id, tokens, max_len + 1, score, steps));
+  if (n_best > 0) {
+    HM_TRY(beam_finalize(st, state, p.bm_score, p.bp_parent, p.bp_token, p.bp_logp, B, beam, n_best, rows, max_len,
+                         e->cfg.sos_id, e->cfg.pad_id, tokens, logprob, score, steps));
+  } else if (beam_mode) {
+    HM_TRY(beam_finalize(st, state, p.bm_score, p.bp_parent, p.bp_token, nullptr, B, beam, 1, rows, max_len,
+                         e->cfg.sos_id, e->cfg.pad_id, tokens, nullptr, score, steps));
     if (logprob != nullptr) HM_CUDA(cudaMemsetAsync(logprob, 0, sizeof(float) * B * max_len, st));
   } else {
     HM_TRY(finalize_decode(st, state, tokens, max_len + 1, rows, max_len, e->cfg.pad_id, logprob, steps));
@@ -955,14 +964,14 @@ int encode_for_generate(hmocr_engine* e, const float* images, int B, float* enc3
 }
 
 int generate_impl(hmocr_engine* e, const float* images, int B, int max_len, int beam, int64_t* tokens, float* logprob,
-                  int32_t* steps, float* score, cudaStream_t st) {
+                  int32_t* steps, float* score, cudaStream_t st, int n_best = 0) {
   float* enc32;
   h16* enc16;
   HM_TRY(ws_get(e, "gen.enc32", (size_t)B * e->mem_len * e->cfg.d_model, &enc32));
   HM_TRY(ws_get(e, "gen.enc16", (size_t)B * e->mem_len * e->cfg.d_model, &enc16));
   if (e->planning) {
     HM_TRY(encode_for_generate(e, images, B, enc32, enc16, st));
-    return generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st);
+    return generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
   }
   HM_CUDA(cudaEventRecord(e->ev[0], st));
   nvtx_push("hmocr.encode");
@@ -970,7 +979,21 @@ int generate_impl(hmocr_engine* e, const float* images, int B, int max_len, int 
   nvtx_pop();
   HM_TRY(rc_enc);
   HM_CUDA(cudaEventRecord(e->ev[1], st));
-  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st));
+  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
+  HM_CUDA(cudaEventRecord(e->ev[2], st));
+  e->timings_pending = true;
+  return 0;
+}
+
+// generate from encoder output already in HBM (f32 [B, mem_len, d_model])
+int generate_from_enc32(hmocr_engine* e, const float* enc_out, int B, int max_len, int beam, int64_t* tokens,
+                        float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best) {
+  h16* enc16;
+  HM_TRY(ws_get(e, "gen.enc16", (size_t)B * e->mem_len * e->cfg.d_model, &enc16));
+  HM_TRY(f32_to_f16(st, enc_out, (size_t)B * e->mem_len * e->cfg.d_model, enc16));
+  HM_CUDA(cudaEventRecord(e->ev[0], st));
+  HM_CUDA(cudaEventRecord(e->ev[1], st));
+  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
   HM_CUDA(cudaEventRecord(e->ev[2], st));
   e->timings_pending = true;
   return 0;
@@ -994,6 +1017,8 @@ int plan_workspace(hmocr_engine* e, int B, int max_len, int beam, size_t* bytes)
   int64_t* tdummy = reinterpret_cast<int64_t*>(WS_ALIGN);
   if (beam == 0) {                                   // teacher-forced hmocr_decoder_forward(B, T = max_len)
     rc = decoder_forward_impl(e, fdummy, tdummy, B, max_len, fdummy, nullptr);
+  } else if (beam < 0) {                             // hmocr_generate_nbest with -beam hypotheses (either input form)
+    rc = generate_impl(e, fdummy, B, max_len, -beam, tdummy, fdummy, nullptr, fdummy, nullptr, 1);
   } else {                                           // hmocr_encode + hmocr_generate* (device and host-buffer forms)
     h16* d16;
     uint8_t* u8;
@@ -1232,7 +1257,7 @@ HM_API int hmocr_set_pos_table(hmocr_engine* e, const float* pos_host, int rows,
 HM_API int hmocr_workspace_bytes(hmocr_engine* e, int batch, int max_len, int beam, size_t* bytes) {
   HM_CHECK(e != nullptr && bytes != nullptr, "hmocr_workspace_bytes: null argument");
   HM_CHECK(e->finalized, "hmocr_workspace_bytes: load the weights first (buffer sizes depend on the checkpoint's vocabulary)");
-  HM_CHECK(batch >= 1 && max_len >= 1 && beam >= 0, "hmocr_workspace_bytes: bad shape batch=%d max_len=%d beam=%d", batch, max_len, beam);
+  HM_CHECK(batch >= 1 && max_len >= 1 && beam >= -DP_MAX_BEAM, "hmocr_workspace_bytes: bad shape batch=%d max_len=%d beam=%d", batch, max_len, beam);
   return plan_workspace(e, batch, max_len, beam, bytes);
 }
 
@@ -1330,16 +1355,19 @@ HM_API int hmocr_generate_from_memory(hmocr_engine* e, const float* enc_out, int
                                       int64_t* tokens, float* logprob, int32_t* steps, float* score, void* stream) {
   HM_TRY(check_ready(e, B, stream));
   HM_CHECK(enc_out != nullptr && tokens != nullptr, "hmocr_generate_from_memory: null buffer");
+  return generate_from_enc32(e, enc_out, B, max_len, beam, tokens, logprob, steps, score,
+                             static_cast<cudaStream_t>(stream), 0);
+}
+
+HM_API int hmocr_generate_nbest(hmocr_engine* e, const float* input, int input_is_memory, int B, int max_len, int beam,
+                                int n_best, int64_t* tokens, float* logprob, float* score, int32_t* steps, void* stream) {
+  HM_TRY(check_ready(e, B, stream));
+  HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "hmocr_generate_nbest: beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
+  HM_CHECK(n_best >= 1 && n_best <= beam, "hmocr_generate_nbest: n_best=%d outside [1, beam=%d]", n_best, beam);
+  HM_CHECK(input != nullptr && tokens != nullptr, "hmocr_generate_nbest: null buffer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  h16* enc16;
-  HM_TRY(ws_get(e, "gen.enc16", (size_t)B * e->mem_len * e->cfg.d_model, &enc16));
-  HM_TRY(f32_to_f16(st, enc_out, (size_t)B * e->mem_len * e->cfg.d_model, enc16));
-  HM_CUDA(cudaEventRecord(e->ev[0], st));
-  HM_CUDA(cudaEventRecord(e->ev[1], st));
-  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st));
-  HM_CUDA(cudaEventRecord(e->ev[2], st));
-  e->timings_pending = true;
-  return 0;
+  if (input_is_memory) return generate_from_enc32(e, input, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
+  return generate_impl(e, input, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
 }
 
 HM_API int hmocr_generate_host(hmocr_engine* e, const float* images_host, int B, int max_len, int beam,

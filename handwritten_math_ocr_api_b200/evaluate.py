@@ -10,6 +10,9 @@ batch, ``:79``).  The METRICS are kept exactly as the reference computes them (`
 
 Ground truth of a sample = ``captions[i][1 : lengths[i] - 1]`` mapped through ``idx2char`` and joined with spaces
 (``:74-75``).  Predictions come from ``inference.predict`` = ONE ``generate`` call per batch.
+
+With ``n_best > 1`` each row also gets ``in_top_n`` (the truth is among the strings of the ``n_best`` best beam
+hypotheses, one more ``generate_nbest`` call per batch) and the summary ``top_n_accuracy``.
 """
 from __future__ import annotations
 
@@ -41,18 +44,30 @@ def summarize(rows: List[dict]) -> dict:
     }
 
 
+def top_n_strings(model, images, n_best: int, beam_size: int, idx2char: Dict[int, str], config=_default_config):
+    """Per image, the strings of its ``n_best`` best beam hypotheses (beam width ``max(beam_size, n_best)``)."""
+    tokens, _, _, _ = model.generate_nbest(images, beam_size=max(beam_size, n_best), n_best=n_best,
+                                           max_len=config.max_seq_len)
+    B, n, L = tokens.shape
+    flat = inference.ids_to_strings(tokens.reshape(B * n, L).tolist(), idx2char, config)
+    return [flat[b * n:(b + 1) * n] for b in range(B)]
+
+
 def evaluate_model(model, batches: Iterable, vocab, idx2char, device=None, use_beam: bool = False,
-                   beam_size: Optional[int] = None, image_ids: Optional[Iterable] = None, config=_default_config):
+                   beam_size: Optional[int] = None, image_ids: Optional[Iterable] = None, config=_default_config,
+                   n_best: int = 1):
     """``evaluate_model`` (``src/test_model.py:60-87``) over an iterable of ``(images, captions, lengths)`` batches
     (what ``data_loader.get_test_loader`` yields).  Returns ``(rows, summary)``; ``rows`` are dicts with the
-    reference's columns (``image_id`` is the running sample index unless ``image_ids`` supplies one per sample)."""
+    reference's columns (``image_id`` is the running sample index unless ``image_ids`` supplies one per sample).
+    ``n_best > 1`` adds ``in_top_n`` to every row and ``top_n_accuracy`` to the summary."""
     model.eval()
     ids = iter(image_ids) if image_ids is not None else None
+    beam = beam_size if beam_size is not None else config.beam_size
     rows: List[dict] = []
     for images, captions, lengths in batches:
-        preds = inference.predict(images, model, vocab, idx2char, device,
-                                  beam_size=beam_size if beam_size is not None else config.beam_size,
-                                  config=config, use_beam=use_beam)
+        preds = inference.predict(images, model, vocab, idx2char, device, beam_size=beam, config=config,
+                                  use_beam=use_beam)
+        tops = top_n_strings(model, images, n_best, beam, idx2char, config) if n_best > 1 else None
         caps = captions.tolist() if hasattr(captions, "tolist") else captions
         lens = lengths.tolist() if hasattr(lengths, "tolist") else lengths
         for i, pred in enumerate(preds):
@@ -65,4 +80,9 @@ def evaluate_model(model, batches: Iterable, vocab, idx2char, device=None, use_b
                 'is_correct': correct,
                 'cer': cer,
             })
-    return rows, summarize(rows)
+            if tops is not None:
+                rows[-1]['in_top_n'] = truth in tops[i]
+    summary = summarize(rows)
+    if n_best > 1:
+        summary['top_n_accuracy'] = sum(r['in_top_n'] for r in rows) / len(rows) if rows else 0.0
+    return rows, summary

@@ -7,6 +7,9 @@ log-softmax, from which the confidence is rebuilt with the reference's exact boo
 sum of ``log(p + 1e-10)`` over every step INCLUDING the eos step, divided by the number of
 non-eos tokens (im2latex.py:33-39,50,55).  ``predict_batch`` is the tensor-batched form of the
 ``/predict/batch`` Python loop (app/src/main.py:546-550).
+
+``beam_size > 1`` decodes with beam search instead (the reference app's ``DEFAULT_BEAM_SIZE``), and
+``predict_nbest`` returns every image's ranked alternatives, each with the same confidence bookkeeping.
 """
 from __future__ import annotations
 
@@ -61,8 +64,37 @@ def _finish(row_tokens: List[int], row_logp: List[float], eos: int, idx2char) ->
     return formula, float(torch.exp(torch.tensor(lp_sum / len(out_tokens))).item())
 
 
+def rank_hypotheses(tokens, logprobs, scores, eos: int, idx2char) -> List[Tuple[str, float, float]]:
+    """One image's hypotheses, best first (``tokens[j]`` without the sos column, ``logprobs[j]``, ``scores[j]``) ->
+    ``[(formula, confidence, score), ...]``: ``_finish`` on each, and a hypothesis whose formula equals a higher-ranked
+    one's is dropped, so the same formula is never listed twice."""
+    out: List[Tuple[str, float, float]] = []
+    seen = set()
+    for t, lp, sc in zip(tokens, logprobs, scores):
+        formula, conf = _finish(t, lp, eos, idx2char)
+        if formula not in seen:
+            seen.add(formula)
+            out.append((formula, conf, float(sc)))
+    return out
+
+
+def predict_nbest(model, image_tensors: torch.Tensor, vocab: Dict[str, int], idx2char: Dict[int, str],
+                  device: str = "cuda", beam_size: int = 3, n_best: int = 3) -> List[List[Tuple[str, float, float]]]:
+    """Per image, the ranked list of distinct ``(formula, confidence, score)`` among the ``n_best`` best beam
+    hypotheses (``score`` = summed log-probability; entry 0 is ``predict_batch(..., beam_size=beam_size)``)."""
+    model = model.to(device)
+    model.eval()
+    tokens, scores, logp, _ = model.generate_nbest(image_tensors, beam_size=beam_size, n_best=n_best,
+                                                   max_len=config.max_seq_len)
+    toks, lps, scs = tokens[:, :, 1:].cpu().tolist(), logp.cpu().tolist(), scores.cpu().tolist()
+    eos = vocab[config.eos_token]
+    return [rank_hypotheses(t, l, s, eos, idx2char) for t, l, s in zip(toks, lps, scs)]
+
+
 def predict_batch(model, image_tensors: torch.Tensor, vocab: Dict[str, int], idx2char: Dict[int, str],
-                  device: str = "cuda") -> List[Tuple[str, float]]:
+                  device: str = "cuda", beam_size: int = 1) -> List[Tuple[str, float]]:
+    if beam_size > 1:
+        return [hyps[0][:2] for hyps in predict_nbest(model, image_tensors, vocab, idx2char, device, beam_size, 1)]
     model = model.to(device)
     model.eval()
     tokens, steps, logp = model.generate(image_tensors, max_len=config.max_seq_len, return_logprobs=True)
@@ -71,6 +103,6 @@ def predict_batch(model, image_tensors: torch.Tensor, vocab: Dict[str, int], idx
     return [_finish(t, l, eos, idx2char) for t, l in zip(toks, lps)]
 
 
-def predict(model, image_tensor: torch.Tensor, vocab: dict, idx2char: dict, device: str = "cuda"):
+def predict(model, image_tensor: torch.Tensor, vocab: dict, idx2char: dict, device: str = "cuda", beam_size: int = 1):
     """-> (cleaned_formula, confidence_score), im2latex.py:15-56."""
-    return predict_batch(model, image_tensor, vocab, idx2char, device)[0]
+    return predict_batch(model, image_tensor, vocab, idx2char, device, beam_size)[0]

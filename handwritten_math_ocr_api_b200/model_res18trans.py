@@ -82,3 +82,11 @@ class FormulaRecognitionModel(_Base):
             self.set_pos_table(pos_table)
         return super().generate(images, max_len=max_len, beam_size=beam_size, return_logprobs=return_logprobs,
                                 encoder_out=encoder_out)
+
+    @torch.no_grad()
+    def generate_nbest(self, images=None, *, encoder_out=None, beam_size: int = 3, n_best=None, max_len=None,
+                       pos_table: Optional[torch.Tensor] = None):
+        if encoder_out is None:
+            self.set_pos_table(pos_table)
+        return super().generate_nbest(images, encoder_out=encoder_out, beam_size=beam_size, n_best=n_best,
+                                      max_len=max_len)

@@ -12,6 +12,7 @@ Same surface as the reference nn.Module (SURVEY.md section 8b):
 plus the one new entry point the engine exists for:
 
     tokens, steps, logprobs = model.generate(images, max_len=150, beam_size=1)
+    tokens, scores, logprobs, steps = model.generate_nbest(images, beam_size=3)     # ranked beam hypotheses
 
 Every tensor stays a torch CUDA tensor; torch is only the allocator / stream provider.  There is
 no CPU path: ``.to('cpu')`` raises, and a missing ``libhmocr.so`` raises at construction.
@@ -148,7 +149,7 @@ class FormulaRecognitionModel:
         self._n_params = 0
         # scratch memory is a torch tensor handed to the engine (SURVEY.md 8b "Ownership"): see _reserve
         self._workspace: Optional[torch.Tensor] = None
-        self._reserved = {"gen": (0, 0, 0), "tf": (0, 0)}
+        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0)}
         self.encoder = EncoderSwin(self)
         self.decoder = DecoderTransformer(self)
         self.training = False
@@ -256,8 +257,8 @@ class FormulaRecognitionModel:
     def _reserve(self, kind: str, *shape: int) -> None:
         """Make the caller-owned workspace large enough for a call of this shape.
 
-        ``kind='gen'``: ``(batch, max_len, beam)`` of encoder / generate calls; ``kind='tf'``: ``(batch, T)`` of the
-        teacher-forced decoder.  The buffer is ONE uint8 torch tensor (torch's caching allocator, current stream) sized
+        ``kind='gen'``: ``(batch, max_len, beam)`` of encoder / generate calls; ``kind='nbest'``: ``(batch, max_len,
+        beam)`` of generate_nbest calls; ``kind='tf'``: ``(batch, T)`` of the teacher-forced decoder.  The buffer is ONE uint8 torch tensor (torch's caching allocator, current stream) sized
         by ``hmocr_workspace_bytes`` for the largest shapes seen so far and handed over with ``hmocr_set_workspace``;
         the engine allocates nothing itself.  Growing re-places every buffer (rare: shapes only ever grow)."""
         have = self._reserved[kind]
@@ -271,6 +272,9 @@ class FormulaRecognitionModel:
             if kind == "gen":
                 b, t, k = self._reserved["gen"]
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, k, C.byref(n)), "hmocr_workspace_bytes")
+            elif kind == "nbest":
+                b, t, k = self._reserved["nbest"]
+                _lib.check(lib.hmocr_workspace_bytes(h, b, t, -k, C.byref(n)), "hmocr_workspace_bytes")
             else:
                 b, t = self._reserved["tf"]
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, 0, C.byref(n)), "hmocr_workspace_bytes")
@@ -371,6 +375,34 @@ class FormulaRecognitionModel:
         return tokens[:, : n + 1], n, out_lp
 
     @torch.no_grad()
+    def generate_nbest(self, images: Optional[torch.Tensor] = None, *, encoder_out: Optional[torch.Tensor] = None,
+                       beam_size: int = 3, n_best: Optional[int] = None, max_len: Optional[int] = None):
+        """The ``n_best`` (default ``beam_size``) best hypotheses of a beam search per image, ranked by score.
+
+        Returns ``(tokens int64 [B, n, 1+steps], scores f32 [B, n], logprobs f32 [B, n, steps], steps)``.  Rank 0 is
+        what ``generate(beam_size=beam_size)`` returns; ``logprobs`` holds each emitted token's log-softmax (0 after the
+        hypothesis' eos) and ``scores`` is its fp32 sum in step order.  ``beam_size=1`` gives the greedy sequence."""
+        beam = int(beam_size)
+        n = beam if n_best is None else int(n_best)
+        max_len = int(max_len if max_len is not None else self.max_seq_len)
+        x = self._images(images) if encoder_out is None else self._memory(encoder_out)
+        B = x.shape[0]
+        if not 1 <= max_len <= self.max_seq_len:
+            raise RuntimeError(f"max_len={max_len} outside [1, {self.max_seq_len}] (size of pos_encoder, src/model_swin.py:54)")
+        if 1 <= beam <= 5:                      # otherwise the library call below names the problem
+            self._reserve("nbest", B, max_len, beam)
+        tokens = torch.empty(B, max(n, 0), max_len + 1, dtype=torch.int64, device=self.device)
+        logp = torch.empty(B, max(n, 0), max_len, dtype=torch.float32, device=self.device)
+        scores = torch.empty(B, max(n, 0), dtype=torch.float32, device=self.device)
+        steps = torch.zeros(1, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._eng.lib.hmocr_generate_nbest(self._handle(), _ptr(x), int(encoder_out is not None), B,
+                                                          max_len, beam, n, _ptr(tokens), _ptr(logp), _ptr(scores),
+                                                          _ptr(steps), _stream()), "hmocr_generate_nbest")
+        t = int(steps.item())
+        return tokens[:, :, : t + 1], scores, logp[:, :, :t], t
+
+    @torch.no_grad()
     def pack_tokens(self, tokens: torch.Tensor):
         """Detokenise on the device (the per-id Python loop of /root/reference/src/inference.py:29-40): drops sos /
         pad ids, stops at the first eos.  ``tokens`` int64 ``[B, L]`` (CUDA) -> ``(packed int32 [B, L], lengths int32
@@ -389,7 +421,7 @@ class FormulaRecognitionModel:
         include/hmocr.h lists them)."""
         _lib.check(self._eng.lib.hmocr_set_option(self._eng.handle, name.encode(), int(value)), "hmocr_set_option")
         # options change which scratch buffers a call uses (step graph / beam kernel / tracing): plan again
-        self._reserved = {"gen": (0, 0, 0), "tf": (0, 0)}
+        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0)}
 
     def last_decode_steps(self) -> int:
         """Decode steps the persistent kernel executed in the last ``generate`` call (after a stream synchronise): the

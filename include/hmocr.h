@@ -98,7 +98,8 @@ int hmocr_set_pos_table(hmocr_engine* e, const float* pos_host, int rows, int d,
  * activations live in torch's caching allocator, which is where this buffer comes from on the Python side).
  *   hmocr_workspace_bytes: bytes of scratch that hmocr_encode + hmocr_generate* (device and host-buffer forms) need
  *     for `batch` images, `max_len` steps and `beam` hypotheses with the engine's current options; beam == 0 asks for
- *     the teacher-forced hmocr_decoder_forward(batch, T = max_len) instead.  The engine remembers the per-buffer
+ *     the teacher-forced hmocr_decoder_forward(batch, T = max_len) instead, beam < 0 for hmocr_generate_nbest with
+ *     -beam hypotheses.  The engine remembers the per-buffer
  *     maximum over all shapes asked so far, and *bytes covers ALL of them (ask once per shape you will use, pass the
  *     last answer to hmocr_set_workspace).
  *   hmocr_set_workspace: hand the engine one device buffer (256-byte aligned).  It stays the caller's; it must
@@ -140,6 +141,23 @@ int hmocr_generate(hmocr_engine* e, const float* images_dev, int batch, int max_
 int hmocr_generate_from_memory(hmocr_engine* e, const float* enc_out_dev, int batch, int max_len, int beam,
                                int64_t* tokens_dev, float* logprob_dev, int32_t* steps_dev, float* score_dev,
                                void* stream);
+
+/* The n best hypotheses of a beam search, ranked, with per-token log-probabilities ("did you mean ..." alternatives).
+ * Always runs the beam-search machinery, 1 <= beam <= 5 (beam == 1 gives the greedy sequence, padded after eos,
+ * with its score); 1 <= n_best <= beam, otherwise the call fails with a message.
+ *   input_dev     images f32 [B,1,96,320] (input_is_memory == 0) or encoder output f32 [B,mem_tokens,d_model] (!= 0)
+ *   tokens_dev    int64 [B, n_best, 1+max_len]  hypotheses by score, highest first (ties -> lower beam index, so rank 0
+ *                                               is exactly what hmocr_generate returns); column 0 = sos, pad after a
+ *                                               hypothesis' eos and past *steps
+ *   logprob_dev   f32   [B, n_best, max_len]    log_softmax of each emitted token, 0 after eos and past *steps
+ *                                               (may be NULL)
+ *   score_dev     f32   [B, n_best]             summed log-probability = the fp32 sum of the row of logprob_dev in step
+ *                                               order (may be NULL)
+ *   steps_dev     int32 [1]                     decode steps executed (may be NULL)
+ * The workspace of a call with `beam` hypotheses is sized by hmocr_workspace_bytes(batch, max_len, -beam). */
+int hmocr_generate_nbest(hmocr_engine* e, const float* input_dev, int input_is_memory, int batch, int max_len, int beam,
+                         int n_best, int64_t* tokens_dev, float* logprob_dev, float* score_dev, int32_t* steps_dev,
+                         void* stream);
 
 /* End-to-end form with HOST buffers (what `predict(images, model, vocab, idx2char, device)` does
  * around the model: images.to(device) ... ids back on the host): pinned or pageable host memory
