@@ -641,6 +641,9 @@ int generate_from_memory_impl(hmocr_engine* e, const h16* enc16, int B, int max_
   HM_CHECK(max_len >= 1 && max_len <= e->cfg.max_seq_len,
            "max_len=%d outside [1, %d] (size of pos_encoder, src/model_swin.py:54)", max_len, e->cfg.max_seq_len);
   HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
+  // The beam kernel merges per-hypothesis top-`beam` token lists; with fewer tokens than hypotheses a list has empty
+  // slots, and the candidate built from one (hyp * vocab + 0x7fffffff) overflows into a negative parent index.
+  HM_CHECK(beam <= e->cfg.vocab_size, "beam=%d exceeds vocab_size=%d", beam, e->cfg.vocab_size);
   if (e->decode_impl == 0 || n_best > 0)
     return generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
   HM_CHECK(beam == 1, "the step-graph decode (decode_impl=1) is greedy only; beam=%d needs decode_impl=0", beam);

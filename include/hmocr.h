@@ -133,7 +133,8 @@ int hmocr_decoder_forward(hmocr_engine* e, const float* enc_out_dev, const int64
  * beam  > 1: beam search (2..5 hypotheses per image) as defined in DESIGN.md section 4.5 - the reference
  *            has none, `beam_size` is an unused parameter of src/inference.py:7; tokens are the best
  *            hypothesis per image (finished hypotheses are padded), score_dev f32 [B] its summed
- *            log-probability (may be NULL); logprob_dev is zero-filled. */
+ *            log-probability (may be NULL); logprob_dev is zero-filled.  beam must not exceed vocab_size (a
+ *            step keeps `beam` distinct tokens per hypothesis); a larger beam fails with a message. */
 int hmocr_generate(hmocr_engine* e, const float* images_dev, int batch, int max_len, int beam, int64_t* tokens_dev,
                    float* logprob_dev, int32_t* steps_dev, float* score_dev, void* stream);
 
@@ -144,7 +145,7 @@ int hmocr_generate_from_memory(hmocr_engine* e, const float* enc_out_dev, int ba
 
 /* The n best hypotheses of a beam search, ranked, with per-token log-probabilities ("did you mean ..." alternatives).
  * Always runs the beam-search machinery, 1 <= beam <= 5 (beam == 1 gives the greedy sequence, padded after eos,
- * with its score); 1 <= n_best <= beam, otherwise the call fails with a message.
+ * with its score), beam <= vocab_size; 1 <= n_best <= beam, otherwise the call fails with a message.
  *   input_dev     images f32 [B,1,96,320] (input_is_memory == 0) or encoder output f32 [B,mem_tokens,d_model] (!= 0)
  *   tokens_dev    int64 [B, n_best, 1+max_len]  hypotheses by score, highest first (ties -> lower beam index, so rank 0
  *                                               is exactly what hmocr_generate returns); column 0 = sos, pad after a

@@ -147,7 +147,9 @@ def beam_search(enc: torch.Tensor, sd: SD, cfg: ModelConfig, beam: int, max_len:
     * stop after ``max_len`` steps or when every hypothesis of every image is finished;
     * result per image = highest-score hypothesis (ties -> lowest index), no length penalty.
 
-    -> (tokens int64 [B, 1+steps] best hypothesis, scores f32 [B], all_tokens [B,beam,1+steps],
+    Scores and log-probabilities are computed in the dtype of ``enc`` (float64 inputs give a float64 search).
+
+    -> (tokens int64 [B, 1+steps] best hypothesis, scores [B], all_tokens [B,beam,1+steps],
         all_scores [B,beam])
     """
     B, V = enc.shape[0], cfg.vocab_size
@@ -156,15 +158,15 @@ def beam_search(enc: torch.Tensor, sd: SD, cfg: ModelConfig, beam: int, max_len:
     dec = CachedDecoder(enc, sd, cfg)
     mem_index = torch.arange(B, device=dev).repeat_interleave(beam)
     seqs = torch.full((B, beam, 1), cfg.sos, dtype=torch.long, device=dev)
-    scores = torch.full((B, beam), float("-inf"), device=dev)
+    scores = torch.full((B, beam), float("-inf"), device=dev, dtype=enc.dtype)
     scores[:, 0] = 0.0
     finished = torch.zeros(B, beam, dtype=torch.bool, device=dev)
     for _ in range(max_len):
         logits = dec.step(seqs[:, :, -1].reshape(-1), mem_index)                  # [B*beam, V]
-        logp = torch.log_softmax(logits.float(), -1).reshape(B, beam, V)
+        logp = torch.log_softmax(logits.to(enc.dtype), -1).reshape(B, beam, V)
         cand = scores.unsqueeze(-1) + logp
         # finished hypotheses: single candidate (pad) with the frozen score
-        fin_row = torch.full((V,), float("-inf"), device=dev)
+        fin_row = torch.full((V,), float("-inf"), device=dev, dtype=enc.dtype)
         fin_row[cfg.pad] = 0.0
         cand = torch.where(finished.unsqueeze(-1), scores.unsqueeze(-1) + fin_row, cand)
         flat = cand.reshape(B, beam * V)
