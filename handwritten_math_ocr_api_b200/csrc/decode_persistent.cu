@@ -471,13 +471,11 @@ __device__ __forceinline__ float chunk_bias(const uint8_t* slot, int r) {
 }
 
 // KB = 0: greedy.  KB = DP_MAX_BEAM: beam search with p.beam <= KB hypotheses per image (see decode_persistent.cuh).
-// DEV = true: the instrumented build (phase tracing, the timing-experiment flags); the production instantiations
-// carry none of that code.
+// DEV = true: the instrumented build (phase tracing); the production instantiations carry none of that code.
 template <int NB, int KB, bool DEV>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(THREADS, 2)
 decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
   constexpr bool BEAM = KB > 0;
-  const int dev_flags = DEV ? p.flags : 0;
   extern __shared__ __align__(128) uint8_t smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -512,8 +510,7 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
       bulk_g2s(s.slot[warp], wst + (size_t)wpos * DP_CHUNK, DP_CHUNK, &s.full[warp]);
     }
   };
-  const bool dbg_noweights = (dev_flags & 4) != 0;      // timing experiments only (results are wrong)
-  auto slot_wait = [&]() { if (!dbg_noweights || wk == 0) mbar_wait_trap(&s.full[warp], wk & 1); };
+  auto slot_wait = [&]() { mbar_wait_trap(&s.full[warp], wk & 1); };
   auto slot_release = [&]() {
     __syncwarp();
     // The warp has read the slot through the generic proxy (ldmatrix, the bias words); the refill below writes it
@@ -524,7 +521,7 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
     fence_proxy_async();
     ++wk; wgi += NW; wpos += NW;
     if (wpos >= S) wpos -= S;
-    if (lane == 0 && !dbg_noweights) slot_fetch();
+    if (lane == 0) slot_fetch();
   };
   // ---- exchanges --------------------------------------------------------------------------------------
   // The mbarrier phase parities follow from two counters instead of one per exchange: per layer the context barrier
@@ -692,7 +689,7 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
       __half* Vd = p.vcache + set_wr + (size_t)l * kv_layer + kv_row;
       TR();
       // ---- self-attention: q, k, v of head c = 6 tiles ---------------------------------------------
-      if (lane < 2 && !(dev_flags & 2)) prefetch_l2<true>((lane ? p.memv : p.memk) + (size_t)l * m_layer + m_row, region_bytes(p.mem_len));   // this layer's memory K/V -> L2
+      if (lane < 2) prefetch_l2<true>((lane ? p.memv : p.memk) + (size_t)l * m_layer + m_row, region_bytes(p.mem_len));   // this layer's memory K/V -> L2
       {
         const int j = (warp - g) & 7;
         if (j < 6) {
@@ -716,14 +713,13 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
         g += 6;
       }
       KvPair kv;
-      const int nhist = (dev_flags & 8) ? min(t, 1) : t;
-      attend_issue2<false>(Kc, Vc, nhist, lane, kv);           // the first K and V block fly across the barrier
+      attend_issue2<false>(Kc, Vc, t, lane, kv);           // the first K and V block fly across the barrier
       TR();
       __syncthreads();
       TR();
       {
         float o[4];
-        attend_online<NB, true, BEAM, false>(&s.qh[warp][0], Kc, Vc, nhist, &s.knew[warp][0], &s.vnew[warp][0],
+        attend_online<NB, true, BEAM, false>(&s.qh[warp][0], Kc, Vc, t, &s.knew[warp][0], &s.vnew[warp][0],
                                              lane, kv, o, row_ok ? Kd : nullptr, row_ok ? Vd : nullptr);   // padding warps
         // recompute the last valid row: they must not copy its blocks (a late copy would overwrite the append below)
         TR();
@@ -737,7 +733,7 @@ decode_persistent_kernel(const DecPersistParams p, int t_begin, int t_end) {
         // beam search the parent row is not known a step ahead (the beam kernel is 2 % faster without it).
         const bool last = l + 1 == L;
         const int keys = last ? t + 1 : t;
-        if (!BEAM && keys > 0 && lane < 2 && !(dev_flags & 1)) {
+        if (!BEAM && keys > 0 && lane < 2) {
           const size_t nxt = last ? set_wr + kv_row : set_rd + (size_t)(l + 1) * kv_layer + kv_src;
           prefetch_l2<false>((lane ? p.vcache : p.kcache) + nxt, region_bytes(keys));
         }
@@ -1202,7 +1198,7 @@ int decode_persistent_launch(cudaStream_t st, DecPersistParams p, int t_begin, i
   HM_CHECK(p.cache_blocks * 32 >= p.tmax, "decode: %d cache blocks cannot hold %d positions", p.cache_blocks, p.tmax);
   HM_CHECK(p.mem_len >= 1 && p.mem_len <= 32, "decode: %d memory tokens per image (1..32 supported)", p.mem_len);
   HM_CHECK(p.beam >= 1 && p.beam <= DP_MAX_BEAM, "decode: beam %d outside [1, %d]", p.beam, DP_MAX_BEAM);
-  const bool beam = p.beam > 1 || p.bm_score != nullptr;     // beam machinery (also runs beam = 1 for the A/B test)
+  const bool beam = p.beam > 1 || p.bm_score != nullptr;     // beam machinery (n-best runs it at beam = 1 too)
   // Rows per cluster: 8 (greedy) or whole images (beam).  Clusters are independent, so a batch larger than
   // rows_per_cluster x (co-resident clusters) simply runs in several waves.
   if (beam) {
@@ -1213,9 +1209,8 @@ int decode_persistent_launch(cudaStream_t st, DecPersistParams p, int t_begin, i
   }
   p.num_clusters = ceil_div(p.rows, p.rows_per_cluster);
   dim3 grid(p.num_clusters * CL);
-  const bool dev = p.trace != nullptr || p.flags != 0;       // instrumented build: greedy, <= 160 positions only
-  if (dev) {
-    HM_CHECK(!beam && p.tmax <= 160, "decode: tracing / experiment flags need greedy decoding and max_seq_len <= 160");
+  if (p.trace != nullptr) {                                  // instrumented build: greedy, <= 160 positions only
+    HM_CHECK(!beam && p.tmax <= 160, "decode: tracing needs greedy decoding and max_seq_len <= 160");
     decode_persistent_kernel<5, 0, true><<<grid, THREADS, sizeof(Smem), st>>>(p, t_begin, t_end);
   } else if (p.tmax <= 160) {
     if (beam) decode_persistent_kernel<5, DP_MAX_BEAM, false><<<grid, THREADS, sizeof(Smem), st>>>(p, t_begin, t_end);

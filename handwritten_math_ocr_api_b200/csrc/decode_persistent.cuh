@@ -64,7 +64,6 @@ struct DecPersistParams {
   int tmax, max_pos, max_len, ld_tok, eos, pad;
   long long* trace;           // optional: clock64() of cluster 0 / CTA 0 / thread 0 at every phase boundary
   int trace_step;             //           of decode step `trace_step`
-  int flags;                  // developer switches: 1 = no L2 prefetch of the next layer's cache, 2 = none of the memory K/V
 };
 
 int decode_persistent_init();

@@ -104,9 +104,7 @@ struct hmocr_engine {
   int decode_impl = 0;                // 0 = persistent cluster kernel, 1 = per-kernel step graph
   int steps_per_launch = 0;           // 0 = automatic (see generate_persistent)
   int trace_step = -1;                // >= 0: record phase-boundary clocks of that decode step
-  int dbg_flags = 0;                  // DecPersistParams::flags
   int conv_impl = 0;                  // ResNet trunk: 0 = implicit GEMM (TMA patches), 1 = explicit im2col + GEMM
-  int force_beam_kernel = 0;          // run beam = 1 through the beam-search kernel (A/B test against greedy)
   int mlp_fused = 1;                  // Swin stages 1/2: fc1 + GELU + fc2 + residual in one kernel (0 = two GEMM launches)
 
   // Scratch buffers, addressed by name; any (re)placement invalidates the captured graphs (ws_epoch).
@@ -800,12 +798,12 @@ int pack_decode_operands(hmocr_engine* e) {
 
 // decode with the persistent cluster kernel: a few launches of `steps_per_launch` steps, the host only polls
 // the all-finished flag of the PREVIOUS launch (the GPU never idles).  beam == 1: greedy
-// (src/inference.py:15-25).  beam > 1 (or option "force_beam_kernel"): beam search as defined in
+// (src/inference.py:15-25).  beam > 1 (or n_best > 0, at any beam): beam search as defined in
 // oracle/decode.py::beam_search - rows = images x beam hypotheses, two K/V cache sets, back-track at the end.
 int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam, int64_t* tokens,
                         float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best) {
   const int nh = e->cfg.nhead, L = e->cfg.num_layers, rows = B * beam;
-  const bool beam_mode = beam > 1 || e->force_beam_kernel || n_best > 0;
+  const bool beam_mode = beam > 1 || n_best > 0;
   HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
   float* memkv;                       // memory K/V of all layers, fp32 out of the GEMM, fp16 after the repack
   __half *memk, *memv, *kcache, *vcache;
@@ -861,7 +859,7 @@ int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, i
   p.chunks_per_step = e->dp_chunks_per_step;
   p.vocab = e->cfg.vocab_size; p.tmax = tmax; p.max_pos = e->cfg.max_seq_len; p.max_len = max_len;
   p.ld_tok = max_len + 1; p.eos = e->cfg.eos_id; p.pad = e->cfg.pad_id; p.cache_blocks = cache_blocks; p.mem_len = e->mem_len;
-  p.trace_step = e->trace_step; p.flags = e->dbg_flags;
+  p.trace_step = e->trace_step;
   p.rows_per_cluster = DP_ROWS;
   if (beam_mode) {
     p.rows_per_cluster = beam * (DP_ROWS / beam);
@@ -1305,12 +1303,8 @@ HM_API int hmocr_set_option(hmocr_engine* e, const char* name, int value) {
   } else if (n == "conv_impl") {
     HM_CHECK(value == 0 || value == 1, "conv_impl must be 0 (implicit GEMM) or 1 (im2col)");
     e->conv_impl = value;
-  } else if (n == "dbg_flags") {
-    e->dbg_flags = value;
   } else if (n == "gemm_dbg") {
     gemm_set_debug(value);
-  } else if (n == "force_beam_kernel") {
-    e->force_beam_kernel = value != 0;
   } else if (n == "mlp_fused") {
     HM_CHECK(value == 0 || value == 1, "mlp_fused must be 0 (fc1 and fc2 as two GEMM launches) or 1 (one kernel)");
     if (e->mlp_fused != value) ++e->ws_epoch;            // captured encoder graphs hold the other schedule

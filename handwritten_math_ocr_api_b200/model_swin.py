@@ -420,7 +420,7 @@ class FormulaRecognitionModel:
         """Engine options of ``hmocr_set_option`` (``decode_impl``, ``steps_per_launch``, ``encoder_graph``, ``mlp_fused``, ...:
         include/hmocr.h lists them)."""
         _lib.check(self._eng.lib.hmocr_set_option(self._eng.handle, name.encode(), int(value)), "hmocr_set_option")
-        # options change which scratch buffers a call uses (step graph / beam kernel / tracing): plan again
+        # options change which scratch buffers a call uses (step graph / tracing): plan again
         self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0)}
 
     def last_decode_steps(self) -> int:

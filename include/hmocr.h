@@ -73,7 +73,6 @@ int hmocr_finalize_weights(hmocr_engine* e);
  *   "steps_per_launch"  decode steps per persistent-kernel launch; 0 (default) = automatic: one launch for the whole
  *                       decode when all clusters of the batch are co-resident (the kernel stops by itself once every
  *                       row has emitted eos), 16-step launches with a host poll in between for multi-wave batches
- *   "force_beam_kernel" 1 = run beam == 1 through the beam-search kernel (A/B test against greedy)
  *   "encoder_graph"     1 (default) = hmocr_generate* replay the encoder's ~95 kernels as one captured CUDA graph for
  *                       batches of up to 1024 images (GPU-side gain in the launch-bound regime of <= 32 images, host-side
  *                       gain beyond; first call at a batch size runs eagerly, the second captures); 0 = always launch
@@ -144,8 +143,9 @@ int hmocr_generate_from_memory(hmocr_engine* e, const float* enc_out_dev, int ba
                                void* stream);
 
 /* The n best hypotheses of a beam search, ranked, with per-token log-probabilities ("did you mean ..." alternatives).
- * Always runs the beam-search machinery, 1 <= beam <= 5 (beam == 1 gives the greedy sequence, padded after eos,
- * with its score), beam <= vocab_size; 1 <= n_best <= beam, otherwise the call fails with a message.
+ * Always runs the beam-search machinery, 1 <= beam <= 5 (beam == 1 runs it with one hypothesis: the greedy sequence,
+ * padded after eos, with its score and per-token log-probabilities), beam <= vocab_size; 1 <= n_best <= beam,
+ * otherwise the call fails with a message.
  *   input_dev     images f32 [B,1,96,320] (input_is_memory == 0) or encoder output f32 [B,mem_tokens,d_model] (!= 0)
  *   tokens_dev    int64 [B, n_best, 1+max_len]  hypotheses by score, highest first (ties -> lower beam index, so rank 0
  *                                               is exactly what hmocr_generate returns); column 0 = sos, pad after a

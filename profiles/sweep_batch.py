@@ -16,15 +16,12 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--batches", default="64,128,256,512")
 ap.add_argument("--max-len", type=int, default=150)
 ap.add_argument("--spl", type=int, default=0, help="steps per persistent-kernel launch (0 = engine default)")
-ap.add_argument("--flags", type=int, default=0, help="decode kernel experiment flags (dbg_flags)")
 a = ap.parse_args()
 cfg = ModelConfig()
 m = FormulaRecognitionModel(cfg.vocab_size)
 m.load_state_dict(synth_state_dict(cfg, seed=0, eos_bias_sigma=0.0))
 if a.spl:
     m.set_option("steps_per_launch", a.spl)
-if a.flags:
-    m.set_option("dbg_flags", a.flags)
 base = synth_images(8, seed=1234).cuda()
 for B in [int(x) for x in a.batches.split(",")]:
     imgs = base.repeat((B + 7) // 8, 1, 1, 1)[:B].contiguous()

@@ -24,7 +24,6 @@ TAIL = ["fc_out tiles + warp reduce + sync", "partials send + wait", "token sele
 ap = argparse.ArgumentParser()
 ap.add_argument("--batch", type=int, default=256)
 ap.add_argument("--step", type=int, default=100)
-ap.add_argument("--flags", type=int, default=0)
 a = ap.parse_args()
 cfg = ModelConfig()
 m = FormulaRecognitionModel(cfg.vocab_size)
@@ -34,7 +33,6 @@ imgs = imgs.repeat((a.batch + 7) // 8, 1, 1, 1)[: a.batch].contiguous()
 enc = m.encoder(imgs)
 m.generate(encoder_out=enc, max_len=150)
 m.set_option("trace_step", a.step)
-m.set_option("dbg_flags", a.flags)
 m.generate(encoder_out=enc, max_len=150)
 torch.cuda.synchronize()
 buf = (C.c_int64 * 1024)()

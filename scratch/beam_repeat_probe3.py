@@ -11,20 +11,19 @@ N = int(sys.argv[1]); NIMG = int(sys.argv[2]); BEAM = int(sys.argv[3]); SPL = in
 GREEDY = BEAM == 0
 if GREEDY:
     BEAM = 1
-elif BEAM == 1:
-    m.set_option("force_beam_kernel", 1)
 if SPL:
     m.set_option("steps_per_launch", SPL)
-FLAGS = int(sys.argv[5]) if len(sys.argv) > 5 else 0
-if FLAGS:
-    m.set_option("dbg_flags", FLAGS)
 imgs = synth_images(8, seed=99).cuda().repeat((NIMG + 7) // 8, 1, 1, 1)[:NIMG].contiguous()
 feats = m.encoder(imgs)
 per_image = [collections.Counter() for _ in range(NIMG)]
 for rep in range(N):
-    out = m.generate(encoder_out=feats, max_len=70, beam_size=BEAM, return_logprobs=(BEAM == 1))
-    sc = out[3] if BEAM > 1 else out[2].sum(1)
+    if GREEDY:
+        sc = m.generate(encoder_out=feats, max_len=70, return_logprobs=True)[2].sum(1)
+    elif BEAM == 1:     # beam 1 through the beam kernel: n-best returns the scores generate() does not
+        sc = m.generate_nbest(encoder_out=feats, beam_size=1, max_len=70)[1][:, 0]
+    else:
+        sc = m.generate(encoder_out=feats, max_len=70, beam_size=BEAM)[3]
     for i, v in enumerate(sc.tolist()):
         per_image[i][v] += 1
 multi = [(i, dict(c)) for i, c in enumerate(per_image) if len(c) > 1]
-print(f"{'greedy kernel ' if GREEDY else ''}beam {BEAM} images {NIMG} spl {SPL} flags {FLAGS}: images with more than one score value: {len(multi)} of {NIMG}; deviating runs: {sum(sum(c.values()) - max(c.values()) for _, c in [(i, per_image[i]) for i in range(NIMG)])}")
+print(f"{'greedy kernel ' if GREEDY else ''}beam {BEAM} images {NIMG} spl {SPL}: images with more than one score value: {len(multi)} of {NIMG}; deviating runs: {sum(sum(c.values()) - max(c.values()) for _, c in [(i, per_image[i]) for i in range(NIMG)])}")

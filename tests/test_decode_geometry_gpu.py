@@ -146,6 +146,22 @@ def _after_eos(tokens):
     return (seen - (body == EOS).int()) > 0
 
 
+def _nbest_beam1_full_width(m, feats, T):
+    """``hmocr_generate_nbest`` at beam 1 into full-width outputs: tokens [B, 1+T], including the pad past ``steps``
+    (``generate_nbest`` slices them off)."""
+    import ctypes as C
+    from handwritten_math_ocr_api_b200 import _lib
+    B = feats.shape[0]
+    m._reserve("nbest", B, T, 1)
+    tok = torch.full((B, 1, T + 1), -7, dtype=torch.int64, device="cuda")
+    steps = torch.zeros(1, dtype=torch.int32, device="cuda")
+    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    _lib.check(m._eng.lib.hmocr_generate_nbest(m._handle(), C.c_void_p(feats.data_ptr()), 1, B, T, 1, 1,
+                                                C.c_void_p(tok.data_ptr()), None, None, C.c_void_p(steps.data_ptr()),
+                                                stream), "hmocr_generate_nbest")
+    return tok[:, 0], int(steps.item())
+
+
 def _sequential_sum(lp):
     acc = torch.zeros(lp.shape[:-1], dtype=torch.float32, device=lp.device)
     for t in range(lp.shape[-1]):
@@ -192,20 +208,16 @@ def test_teacher_forced_logits_every_column(geo):
 
 
 @pytest.mark.parametrize("geo", list(GEOMETRIES))
-def test_beam_kernel_and_step_graph_reproduce_greedy(geo):
-    """``force_beam_kernel`` (beam 1 through the beam build) is the greedy decode, padded after each row's eos;
+def test_beam_one_nbest_and_step_graph_reproduce_greedy(geo):
+    """Beam-1 n-best (beam 1 through the beam build) is the greedy decode, padded after each row's eos;
     the step-graph decode (``decode_impl = 1``) agrees with the persistent kernel up to an fp64 near-tie."""
     g = _geometry(geo)
     m = g.model
     tok, steps, _, _, ref = _greedy(g)
-    m.set_option("force_beam_kernel", 1)
-    try:
-        tb, sb, _ = m.generate_device(encoder_out=g.feats, max_len=g.T)
-    finally:
-        m.set_option("force_beam_kernel", 0)
+    tb, sb = _nbest_beam1_full_width(m, g.feats, g.T)
     want = tok.clone()
     want[:, 1:][_after_eos(tok)] = PAD
-    assert int(sb.item()) == steps and torch.equal(tb, want)
+    assert sb == steps and torch.equal(tb, want)
     m.set_option("decode_impl", 1)
     try:
         t1, s1, _ = m.generate_device(encoder_out=g.feats, max_len=g.T)
@@ -405,9 +417,9 @@ def _tie_engine(V, kind):
 
 
 @pytest.mark.parametrize("V,kind", TIE_CASES)
-def test_exact_ties_greedy(V, kind):
-    """Greedy picks the lowest index of the maximum at every step (torch.argmax), on all three decode paths, and its
-    log-prob is log_softmax(bias)[token]."""
+def test_exact_ties_greedy_on_every_decode_path(V, kind):
+    """Greedy picks the lowest index of the maximum at every step (torch.argmax), on the persistent kernel, the step
+    graph and beam-1 n-best, and its log-prob is log_softmax(bias)[token]."""
     g = _tie_engine(V, kind)
     m, T = g.model, g.T
     top = int(torch.nonzero(g.bias == g.bias.max())[0])
@@ -417,13 +429,14 @@ def test_exact_ties_greedy(V, kind):
     tok, steps, lp = m.generate(encoder_out=g.feats, max_len=T, return_logprobs=True)
     assert steps == T and torch.equal(tok, want)
     assert float((lp.double() - want_lp).abs().max()) < 1e-5
-    for opt in ("decode_impl", "force_beam_kernel"):
-        m.set_option(opt, 1)
-        try:
-            t2, s2, _ = m.generate(encoder_out=g.feats, max_len=T)
-        finally:
-            m.set_option(opt, 0)
-        assert s2 == T and torch.equal(t2, want), opt
+    m.set_option("decode_impl", 1)
+    try:
+        t2, s2, _ = m.generate(encoder_out=g.feats, max_len=T)
+    finally:
+        m.set_option("decode_impl", 0)
+    assert s2 == T and torch.equal(t2, want)
+    tk, _, _, steps = m.generate_nbest(encoder_out=g.feats, beam_size=1, max_len=T)
+    assert steps == T and torch.equal(tk[:, 0], want)
 
 
 @pytest.mark.parametrize("K", [2, 3, 5])

@@ -401,24 +401,6 @@ def _oracle_sequence_score(enc, tokens, sd, cfg):
     return torch.tensor(out)
 
 
-def test_beam_kernel_with_one_hypothesis_equals_greedy(model, cfg, golden_src):
-    """beam = 1 pushed through the beam-search machinery (top-K lists, candidate merge, parent back-track, two
-    cache sets) must reproduce the greedy kernel token for token up to each row's eos."""
-    feats = torch.from_numpy(golden_src["features"]).cuda()
-    g_tok, g_steps, _ = model.generate(encoder_out=feats, max_len=48)
-    model.set_option("force_beam_kernel", 1)
-    try:
-        b_tok, b_steps, _ = model.generate(encoder_out=feats, max_len=48)
-    finally:
-        model.set_option("force_beam_kernel", 0)
-    assert b_steps == g_steps
-    for r in range(feats.shape[0]):
-        row = g_tok[r].tolist()
-        n = row.index(cfg.eos) + 1 if cfg.eos in row else len(row)
-        assert b_tok[r, :n].tolist() == row[:n]
-        assert all(int(x) == cfg.pad for x in b_tok[r, n:])          # finished hypotheses emit pad
-
-
 @pytest.mark.parametrize("beam", [2, 3, 5])
 def test_beam_search_against_the_oracle(model, sd, cfg, golden_src, beam):
     from oracle import decode as odec
