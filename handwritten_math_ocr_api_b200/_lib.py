@@ -39,6 +39,8 @@ SIGNATURES = {
     "hmocr_generate": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_generate_from_memory": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_generate_nbest": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p]),
+    "hmocr_score": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
+    "hmocr_score_workspace_bytes": (_i, [_p, _i, _i, C.POINTER(C.c_size_t)]),
     "hmocr_generate_host": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "hmocr_preprocess_u8": (_i, [_p, _p, _i, _p, _p]),
     "hmocr_pack_tokens": (_i, [_p, _p, _i, _i, _p, _p, _p]),

@@ -2,6 +2,7 @@
 // (teacher-forced and single-step KV-cached), greedy selection with on-device bookkeeping.
 // Follows /root/reference/src/model_swin.py:72-88 and torch.nn.TransformerDecoderLayer
 // (post-LN; MultiheadAttention: 8 heads x 32, scores scaled by 1/sqrt(32), causal -inf mask).
+#include "gemm.cuh"
 #include "kernels.cuh"
 
 namespace hmocr {
@@ -289,6 +290,82 @@ __global__ void __launch_bounds__(256) pack_tokens_kernel(const int64_t* __restr
   if (lane == 0) lengths[r] = n;
 }
 
+// ---- teacher-forced scoring: merge the log-sum-exp partials of gemm_f16_lse -----------------------
+struct LseAcc {
+  float m, s, tv, bv;
+  int bi;
+};
+
+__device__ __forceinline__ void lse_merge(LseAcc& a, const LseAcc& b) {
+  const float mn = fmaxf(a.m, b.m);
+  if (mn != -INFINITY) a.s = a.s * expf(a.m - mn) + b.s * expf(b.m - mn);
+  a.m = mn;
+  a.tv = fmaxf(a.tv, b.tv);                                     // only one partial holds the target
+  if (b.bv > a.bv || (b.bv == a.bv && b.bi < a.bi)) { a.bv = b.bv; a.bi = b.bi; }
+}
+
+constexpr int SCORE_THREADS = 512;
+constexpr int SCORE_MAX_T = 256;
+
+// One block per sequence b, one warp per position t (strided).  Lane i merges partials i, i + 32, ... in that order,
+// then a fixed shuffle tree merges the lanes.  Position t scores tokens[b, t+1]; positions after the first eos among
+// columns 1..T are 0 / pad and are not merged at all.  Thread 0 sums the row in position order.
+__global__ void __launch_bounds__(SCORE_THREADS) score_combine_kernel(const LsePartial* __restrict__ parts, int num_parts,
+                                                                      const int64_t* __restrict__ tokens, int ld_tok,
+                                                                      int T, int eos, int pad,
+                                                                      float* __restrict__ logprob,
+                                                                      float* __restrict__ score,
+                                                                      int32_t* __restrict__ argmax) {
+  __shared__ float s_lp[SCORE_MAX_T];
+  __shared__ int s_last;                                         // last scored position
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid == 0) s_last = T - 1;
+  __syncthreads();
+  if (tid < T && tokens[(size_t)b * ld_tok + tid + 1] == eos) atomicMin(&s_last, tid);
+  __syncthreads();
+  const int last = s_last;
+  for (int t = warp; t < T; t += SCORE_THREADS / 32) {
+    const size_t o = (size_t)b * T + t;
+    if (t > last) {
+      if (lane == 0) {
+        s_lp[t] = 0.f;
+        if (logprob != nullptr) logprob[o] = 0.f;
+        if (argmax != nullptr) argmax[o] = pad;
+      }
+      continue;
+    }
+    LseAcc a{-INFINITY, 0.f, -INFINITY, -INFINITY, 0x7fffffff};
+    const LsePartial* pr = parts + o * num_parts;
+    for (int p = lane; p < num_parts; p += 32) {
+      const float4 x = __ldg(reinterpret_cast<const float4*>(pr + p));
+      const int bi = __ldg(&pr[p].best_idx);
+      lse_merge(a, LseAcc{x.x, x.y, x.z, x.w, bi});
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      LseAcc other;
+      other.m = __shfl_down_sync(0xffffffffu, a.m, off);
+      other.s = __shfl_down_sync(0xffffffffu, a.s, off);
+      other.tv = __shfl_down_sync(0xffffffffu, a.tv, off);
+      other.bv = __shfl_down_sync(0xffffffffu, a.bv, off);
+      other.bi = __shfl_down_sync(0xffffffffu, a.bi, off);
+      if (lane < off) lse_merge(a, other);
+    }
+    if (lane == 0) {
+      const float lp = a.tv - (a.m + logf(a.s));
+      s_lp[t] = lp;
+      if (logprob != nullptr) logprob[o] = lp;
+      if (argmax != nullptr) argmax[o] = a.bi;
+    }
+  }
+  __syncthreads();
+  if (tid == 0 && score != nullptr) {
+    float acc = 0.f;
+    for (int t = 0; t < T; ++t) acc += s_lp[t];
+    score[b] = acc;
+  }
+}
+
 inline int grid_for(size_t n, int block) {
   size_t g = (n + block - 1) / block;
   if (g > 148 * 16) g = 148 * 16;
@@ -374,6 +451,15 @@ int finalize_decode(cudaStream_t st, const DecodeState* state, int64_t* tokens, 
 int copy_logits(cudaStream_t st, const float* src, int ld, int rows, int n_valid, float* dst) {
   const size_t total = (size_t)rows * n_valid;
   copy_logits_kernel<<<grid_for(total, 256), 256, 0, st>>>(src, ld, total, n_valid, dst);
+  HM_LAUNCHED();
+  return 0;
+}
+
+int score_combine(cudaStream_t st, const LsePartial* parts, int num_parts, const int64_t* tokens, int ld_tok, int B,
+                  int T, int eos, int pad, float* logprob, float* score, int32_t* argmax) {
+  HM_CHECK(T >= 1 && T <= SCORE_MAX_T, "score: T=%d outside [1, %d]", T, SCORE_MAX_T);
+  score_combine_kernel<<<B, SCORE_THREADS, 0, st>>>(parts, num_parts, tokens, ld_tok, T, eos, pad, logprob, score,
+                                                    argmax);
   HM_LAUNCHED();
   return 0;
 }

@@ -521,7 +521,8 @@ struct DecBufs {
   float* logits;
 };
 
-int dec_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
+// the activations of the layer stack; logits stays nullptr (hmocr_score keeps no logits)
+int dec_layer_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
   const int d = e->cfg.d_model, ff = e->cfg.dim_feedforward;
   std::string t(tag);
   HM_TRY(ws_get(e, (t + ".x32").c_str(), rows * d, &b->x32));
@@ -530,8 +531,14 @@ int dec_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
   HM_TRY(ws_get(e, (t + ".q").c_str(), rows * d, &b->q));
   HM_TRY(ws_get(e, (t + ".ctx").c_str(), rows * d, &b->ctx));
   HM_TRY(ws_get(e, (t + ".hid").c_str(), rows * ff, &b->hid));
-  HM_TRY(ws_get(e, (t + ".logits").c_str(), rows * e->vpad, &b->logits));
+  b->logits = nullptr;
   return 0;
+}
+
+// the layer-stack activations plus the rows x vpad fp32 logits
+int dec_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
+  HM_TRY(dec_layer_bufs(e, tag, rows, b));
+  return ws_get(e, (std::string(tag) + ".logits").c_str(), rows * e->vpad, &b->logits);
 }
 
 // everything of one decoder layer after the self-attention context is in b.ctx
@@ -566,19 +573,16 @@ int layer_tail(hmocr_engine* e, const DecLayer& L, int l, const DecBufs& b, int 
 // ------------------------------------------------------------------------------------------------
 // teacher-forced decoder       /root/reference/src/model_swin.py:72-88
 // ------------------------------------------------------------------------------------------------
-int decoder_forward_impl(hmocr_engine* e, const float* enc32, const int64_t* tgt, int B, int T, float* logits,
-                         cudaStream_t st) {
+// The layer stack of the teacher-forced paths: memory K/V of all layers, x = embedding[tok[b, t]] + pos[t] for t < T
+// (tok row pitch ld_tok), then the L layers; the last hidden state is in b.x16.  enc32 != nullptr: the memory is the
+// caller's fp32 encoder output and is converted into enc16 first; enc32 == nullptr: enc16 already holds it.
+int decoder_layers(hmocr_engine* e, const float* enc32, h16* enc16, h16* memkv, const int64_t* tok, int ld_tok, int B,
+                   int T, const DecBufs& b, cudaStream_t st) {
   const int d = e->cfg.d_model, nh = e->cfg.nhead;
   const int rows = B * T;
-  h16 *enc16, *memkv;
-  HM_TRY(ws_get(e, "tf.enc16", (size_t)B * e->mem_len * d, &enc16));
-  HM_TRY(ws_get(e, "tf.memkv", (size_t)B * e->mem_len * e->ca_kv.n, &memkv));
-  DecBufs b;
-  HM_TRY(dec_bufs(e, "tf", rows, &b));
-  if (e->planning) return 0;
-  HM_TRY(f32_to_f16(st, enc32, (size_t)B * e->mem_len * d, enc16));
+  if (enc32 != nullptr) HM_TRY(f32_to_f16(st, enc32, (size_t)B * e->mem_len * d, enc16));
   HM_TRY(project_memory(e, enc16, B, memkv, st));
-  HM_TRY(embed_tokens(st, tgt, T, B, T, e->emb, e->pos, d, e->cfg.vocab_size, b.x32, b.x16));
+  HM_TRY(embed_tokens(st, tok, ld_tok, B, T, e->emb, e->pos, d, e->cfg.vocab_size, b.x32, b.x16));
   for (int l = 0; l < e->cfg.num_layers; ++l) {
     const DecLayer& L = e->layers[l];
     GemmEpilogue ei;
@@ -587,6 +591,20 @@ int decoder_forward_impl(hmocr_engine* e, const float* enc32, const int64_t* tgt
     HM_TRY(mha_prefill_self(st, b.qkv, B, T, nh, b.ctx));
     HM_TRY(layer_tail(e, L, l, b, rows, memkv, nullptr, T, st));
   }
+  return 0;
+}
+
+int decoder_forward_impl(hmocr_engine* e, const float* enc32, const int64_t* tgt, int B, int T, float* logits,
+                         cudaStream_t st) {
+  const int d = e->cfg.d_model;
+  const int rows = B * T;
+  h16 *enc16, *memkv;
+  HM_TRY(ws_get(e, "tf.enc16", (size_t)B * e->mem_len * d, &enc16));
+  HM_TRY(ws_get(e, "tf.memkv", (size_t)B * e->mem_len * e->ca_kv.n, &memkv));
+  DecBufs b;
+  HM_TRY(dec_bufs(e, "tf", rows, &b));
+  if (e->planning) return 0;
+  HM_TRY(decoder_layers(e, enc32, enc16, memkv, tgt, T, B, T, b, st));
   GemmEpilogue eo;
   eo.out_f32 = b.logits; eo.ld32 = e->vpad;
   HM_TRY(run_lin(st, b.x16, d, rows, e->fc, eo));
@@ -1000,6 +1018,39 @@ int generate_from_enc32(hmocr_engine* e, const float* enc_out, int B, int max_le
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------
+// teacher-forced scoring of given sequences (hmocr_score): the layer stack of decoder_forward, then fc_out with the
+// log-sum-exp epilogue (per-row partials, no logits buffer) and one combine kernel
+// ------------------------------------------------------------------------------------------------
+int score_impl(hmocr_engine* e, const float* input, int input_is_memory, int B, int T, const int64_t* tokens,
+               float* logprob, float* score, int32_t* argmax, cudaStream_t st) {
+  const int d = e->cfg.d_model;
+  const int rows = B * T, num_parts = e->vpad / LSE_COLS_PER_PART;
+  const size_t mem_n = (size_t)B * e->mem_len * d;
+  h16 *enc16, *memkv;
+  LsePartial* parts;
+  DecBufs b;
+  HM_TRY(ws_get(e, "tf.memkv", (size_t)B * e->mem_len * e->ca_kv.n, &memkv));
+  HM_TRY(dec_layer_bufs(e, "tf", rows, &b));
+  HM_TRY(ws_get(e, "score.partials", (size_t)rows * num_parts, &parts));
+  const float* enc32 = nullptr;
+  if (input_is_memory) {
+    HM_TRY(ws_get(e, "tf.enc16", mem_n, &enc16));
+    enc32 = input;
+  } else {
+    float* enc_out;
+    HM_TRY(ws_get(e, "gen.enc32", mem_n, &enc_out));
+    HM_TRY(ws_get(e, "gen.enc16", mem_n, &enc16));
+    HM_TRY(encode_for_generate(e, input, B, enc_out, enc16, st));     // records the encoder's buffers when planning
+  }
+  if (e->planning) return 0;
+  HM_TRY(decoder_layers(e, enc32, enc16, memkv, tokens, T + 1, B, T, b, st));
+  GemmLse lse;
+  lse.tokens = tokens; lse.ld_tok = T + 1; lse.T = T; lse.n_valid = e->cfg.vocab_size; lse.partials = parts;
+  HM_TRY(gemm_f16_lse(st, b.x16, d, rows, d, e->fc.w, e->fc.n, e->fc.b, lse));
+  return score_combine(st, parts, num_parts, tokens, T + 1, B, T, e->cfg.eos_id, e->cfg.pad_id, logprob, score, argmax);
+}
+
 int check_ready(hmocr_engine* e, int B, void* stream) {
   HM_CHECK(e != nullptr, "null engine");
   HM_CHECK(e->finalized, "weights not loaded: call hmocr_load_weight for every entry, then hmocr_finalize_weights");
@@ -1010,6 +1061,20 @@ int check_ready(hmocr_engine* e, int B, void* stream) {
 }
 
 // every scratch buffer a call with this shape asks for (the schedules run in planning mode: ws_get records, nothing launches)
+// records the per-buffer maximum of the plan just made and answers the bytes that cover every shape asked so far
+int finish_plan(hmocr_engine* e, size_t* bytes) {
+  e->planning = false;
+  for (auto& kv : e->plan) {
+    size_t& m = e->planned[kv.first];
+    if (m < kv.second) m = kv.second;
+  }
+  e->plan.clear();
+  size_t total = 0;
+  for (auto& kv : e->planned) total += kv.second;    // every entry is already rounded to WS_ALIGN
+  *bytes = total + WS_ALIGN;
+  return 0;
+}
+
 int plan_workspace(hmocr_engine* e, int B, int max_len, int beam, size_t* bytes) {
   e->plan.clear();
   e->planning = true;
@@ -1036,15 +1101,19 @@ int plan_workspace(hmocr_engine* e, int B, int max_len, int beam, size_t* bytes)
     if (rc == 0) rc = ws_get(e, "host.score", B, &f32);
     if (rc == 0) rc = generate_impl(e, fdummy, B, max_len, beam, tdummy, fdummy, nullptr, fdummy, nullptr);
   }
-  e->planning = false;
-  for (auto& kv : e->plan) {
-    size_t& m = e->planned[kv.first];
-    if (m < kv.second) m = kv.second;
-  }
+  finish_plan(e, bytes);
+  return rc;
+}
+
+// hmocr_score(B, T) in both input forms
+int plan_score_workspace(hmocr_engine* e, int B, int T, size_t* bytes) {
   e->plan.clear();
-  size_t total = 0;
-  for (auto& kv : e->planned) total += kv.second;    // every entry is already rounded to WS_ALIGN
-  *bytes = total + WS_ALIGN;
+  e->planning = true;
+  float* fdummy = reinterpret_cast<float*>(WS_ALIGN);
+  int64_t* tdummy = reinterpret_cast<int64_t*>(WS_ALIGN);
+  int rc = score_impl(e, fdummy, 1, B, T, tdummy, fdummy, fdummy, nullptr, nullptr);
+  if (rc == 0) rc = score_impl(e, fdummy, 0, B, T, tdummy, fdummy, fdummy, nullptr, nullptr);
+  finish_plan(e, bytes);
   return rc;
 }
 
@@ -1262,6 +1331,13 @@ HM_API int hmocr_workspace_bytes(hmocr_engine* e, int batch, int max_len, int be
   return plan_workspace(e, batch, max_len, beam, bytes);
 }
 
+HM_API int hmocr_score_workspace_bytes(hmocr_engine* e, int batch, int T, size_t* bytes) {
+  HM_CHECK(e != nullptr && bytes != nullptr, "hmocr_score_workspace_bytes: null argument");
+  HM_CHECK(e->finalized, "hmocr_score_workspace_bytes: load the weights first (buffer sizes depend on the checkpoint's vocabulary)");
+  HM_CHECK(batch >= 1 && T >= 1 && T <= e->cfg.max_seq_len, "hmocr_score_workspace_bytes: bad shape batch=%d T=%d", batch, T);
+  return plan_score_workspace(e, batch, T, bytes);
+}
+
 HM_API int hmocr_set_workspace(hmocr_engine* e, void* workspace_dev, size_t bytes, void* stream) {
   HM_CHECK(e != nullptr, "hmocr_set_workspace: null engine");
   HM_CHECK(workspace_dev == nullptr || (reinterpret_cast<uintptr_t>(workspace_dev) % WS_ALIGN == 0 && bytes >= WS_ALIGN),
@@ -1339,6 +1415,16 @@ HM_API int hmocr_decoder_forward(hmocr_engine* e, const float* enc_out, const in
   HM_CHECK(T >= 1 && T <= e->cfg.max_seq_len, "T=%d outside [1,%d] (tgt_mask / pos_encoder size)", T,
            e->cfg.max_seq_len);
   return decoder_forward_impl(e, enc_out, tgt, B, T, logits, static_cast<cudaStream_t>(stream));
+}
+
+HM_API int hmocr_score(hmocr_engine* e, const float* input, int input_is_memory, int B, int T, const int64_t* tokens,
+                       float* logprob, float* score, int32_t* argmax, void* stream) {
+  HM_TRY(check_ready(e, B, stream));
+  HM_CHECK(input != nullptr && tokens != nullptr, "hmocr_score: null buffer");
+  HM_CHECK(logprob != nullptr || score != nullptr || argmax != nullptr, "hmocr_score: every output is NULL");
+  HM_CHECK(T >= 1 && T <= e->cfg.max_seq_len, "hmocr_score: T=%d outside [1,%d] (tgt_mask / pos_encoder size)", T,
+           e->cfg.max_seq_len);
+  return score_impl(e, input, input_is_memory, B, T, tokens, logprob, score, argmax, static_cast<cudaStream_t>(stream));
 }
 
 HM_API int hmocr_generate(hmocr_engine* e, const float* images, int B, int max_len, int beam, int64_t* tokens,

@@ -72,6 +72,7 @@ struct GemmParams {
   ConvGeom cg;        // CONV kernels only
   int dbg;            // timing experiments only: 1 = skip output stores, 2 = skip residual loads, 4 = skip the epilogue math
   GemmEpilogue epi;
+  GemmLse lse;        // LSE kernels only
 };
 int g_gemm_dbg = 0;
 
@@ -322,7 +323,70 @@ __device__ __forceinline__ void epilogue_ln(const GemmEpilogue& e, uint32_t tadd
   }
 }
 
-template <int BN, bool CONV>
+// Log-sum-exp epilogue (gemm_f16_lse): one thread = one row, as tcgen05.ld hands it over.  Each thread folds its
+// chunks (c = c_first, c_first + 2, ...) in column order into one LsePartial and writes only that: the logits never
+// leave the SM.  Inside a chunk the exponentials are summed as a fixed binary tree.
+template <int BN>
+__device__ __forceinline__ void epilogue_lse(const GemmEpilogue& e, const GemmLse& l, uint32_t taddr, int m_base, int M,
+                                             int n0, int c_first, uint32_t release_bar, int n_tile,
+                                             int num_n_tiles) {
+  const int lane = threadIdx.x & 31;
+  const int row = m_base + lane;
+  int target = -1;
+  if (row < M) {
+    const int b = row / l.T, t = row - b * l.T;
+    const long long id = l.tokens[(size_t)b * l.ld_tok + t + 1];
+    target = (id >= 0 && id < l.n_valid) ? (int)id : -1;
+  }
+  float m = -INFINITY, s = 0.f, tv = -INFINITY, bv = -INFINITY;
+  int bi = 0x7fffffff;
+#pragma unroll 1
+  for (int c = c_first; c < BN / 32; c += 2) {
+    const int col0 = n0 + c * 32;
+    uint32_t r[32];
+    tmem_ld32(taddr + c * 32, r);
+    release_accumulator(c + 2 >= BN / 32, release_bar);
+    float v[32];
+    const float4* b4 = reinterpret_cast<const float4*>(e.bias + col0);
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      const float4 bq = __ldg(b4 + q);
+      v[4 * q] = __uint_as_float(r[4 * q]) + bq.x;
+      v[4 * q + 1] = __uint_as_float(r[4 * q + 1]) + bq.y;
+      v[4 * q + 2] = __uint_as_float(r[4 * q + 2]) + bq.z;
+      v[4 * q + 3] = __uint_as_float(r[4 * q + 3]) + bq.w;
+    }
+    float cm = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      if (col0 + j >= l.n_valid) v[j] = -INFINITY;
+      if (col0 + j == target) tv = v[j];
+      cm = fmaxf(cm, v[j]);
+    }
+    int ci = 0;
+#pragma unroll
+    for (int j = 31; j >= 0; --j) ci = (v[j] == cm) ? j : ci;       // lowest column holding the chunk maximum
+    if (cm > bv) { bv = cm; bi = col0 + ci; }                      // strict: an earlier chunk keeps a tie
+    const float mn = fmaxf(m, cm);
+    if (mn != -INFINITY) {
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] = expf(v[j] - mn);
+#pragma unroll
+      for (int w = 16; w >= 1; w >>= 1)
+#pragma unroll
+        for (int j = 0; j < w; ++j) v[j] += v[j + w];
+      s = s * expf(m - mn) + v[0];
+      m = mn;
+    }
+  }
+  if (row < M) {
+    float4* o = reinterpret_cast<float4*>(l.partials + (size_t)row * (2 * num_n_tiles) + 2 * n_tile + c_first);
+    o[0] = make_float4(m, s, tv, bv);
+    o[1] = make_float4(__int_as_float(bi), 0.f, 0.f, 0.f);
+  }
+}
+
+template <int BN, bool CONV, bool LSE = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const GemmParams p) {
@@ -440,6 +504,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       tc_fence_after();
       const int mb = m0 + quarter * 32;
       const int mi = t / p.num_n_tiles, rq = quarter * 32;
+      if constexpr (LSE) {
+        epilogue_lse<BN>(p.epi, p.lse, taddr, mb, p.M, n0, half, smem_u32(&tempty_bar[group]), t % p.num_n_tiles,
+                         p.num_n_tiles);
+        continue;
+      }
       if (p.mode == EPI_LN) {
         const int row = mb + lane;
         if (half == 0) epilogue_ln<BN>(p.epi, taddr, row, row < p.M, n0);   // row statistics: one thread per row
@@ -677,6 +746,29 @@ int launch(cudaStream_t stream, const h16* A, int lda, int M, int K, const h16* 
   return 0;
 }
 
+int launch_lse(cudaStream_t stream, const h16* A, int lda, int M, int K, const h16* W, int N, const float* bias,
+               const GemmLse& lse) {
+  using C = Cfg<LSE_BN>;
+  alignas(64) CUtensorMap tmA, tmB;
+  HM_TRY(get_tensor_map(A, M, K, lda, BM, &tmA));
+  HM_TRY(get_tensor_map(W, N, K, K, LSE_BN, &tmB));
+  GemmParams p;
+  p.M = M; p.N = N; p.K = K;
+  p.num_n_tiles = N / LSE_BN;
+  p.num_tiles = ceil_div(M, BM) * p.num_n_tiles;
+  p.epi = GemmEpilogue{};
+  p.epi.bias = bias;
+  p.mode = EPI_GENERAL;
+  p.dbg = 0;
+  p.cg = ConvGeom{};
+  p.lse = lse;
+  const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
+  HM_CUDA(launch_pdl(gemm_tcgen05_kernel<LSE_BN, false, true>, dim3(grid), dim3(NUM_THREADS), C::SMEM_BYTES, stream, tmA,
+                     tmB, p));
+  HM_LAUNCHED();
+  return 0;
+}
+
 // NHWC fp16 activation [B, H, W, C] as a 4-D tensor (C, W, H, B); box = 64 channels x (tw, th, tn) output pixels
 // visited with the convolution stride.
 std::map<std::tuple<const void*, int, int, int, int, int, int, int, int>, CUtensorMap> g_maps4;
@@ -843,6 +935,8 @@ int gemm_init() {
   HM_CUDA(cudaFuncSetAttribute(gemm_tcgen05_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<64>::SMEM_BYTES));
   HM_CUDA(cudaFuncSetAttribute(gemm_tcgen05_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128>::SMEM_BYTES));
   HM_CUDA(cudaFuncSetAttribute(gemm_tcgen05_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<256>::SMEM_BYTES));
+  HM_CUDA(cudaFuncSetAttribute(gemm_tcgen05_kernel<LSE_BN, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               Cfg<LSE_BN>::SMEM_BYTES));
   g_encode = reinterpret_cast<EncodeTiledFn>(fn);
   g_sms[dev] = prop.multiProcessorCount;
   return 0;
@@ -898,6 +992,21 @@ int gemm_f16(cudaStream_t stream, const h16* A, int lda, int M, int K, const h16
   }
   HM_CHECK(false, "gemm: unsupported tile width %d", bn);
   return -2;
+}
+
+int gemm_f16_lse(cudaStream_t stream, const h16* A, int lda, int M, int K, const h16* W, int N, const float* bias,
+                 const GemmLse& lse) {
+  HM_TRY(gemm_init());
+  HM_CHECK(M > 0 && K > 0 && N > 0 && N % LSE_BN == 0, "gemm_lse: M=%d K=%d, N=%d must be a multiple of %d", M, K, N,
+           LSE_BN);
+  HM_CHECK(K % 8 == 0 && lda % 8 == 0, "gemm_lse: K=%d and lda=%d must be multiples of 8", K, lda);
+  HM_CHECK((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(bias) & 15) == 0,
+           "gemm_lse: operands and bias must be 16-byte aligned");
+  HM_CHECK(bias != nullptr && lse.tokens != nullptr && lse.partials != nullptr, "gemm_lse: null buffer");
+  HM_CHECK(lse.T >= 1 && lse.ld_tok > lse.T && M % lse.T == 0 && lse.n_valid >= 1 && lse.n_valid <= N,
+           "gemm_lse: bad target geometry M=%d T=%d ld_tok=%d n_valid=%d N=%d", M, lse.T, lse.ld_tok, lse.n_valid, N);
+  return launch_lse(stream, A, lda, M, K, W, N, bias, lse);
 }
 
 }  // namespace hmocr

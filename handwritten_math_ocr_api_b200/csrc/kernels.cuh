@@ -58,6 +58,11 @@ int greedy_select(cudaStream_t st, DecodeState* state, const float* logits, int 
                   int64_t* tokens, int ld_tok, float* logprob, int max_len, int eos, uint8_t* finished,
                   const float* emb, const float* pos, int d, int max_pos, float* x32, h16* x16);
 int advance_step(cudaStream_t st, DecodeState* state);
+// teacher-forced scoring: merge the gemm_f16_lse partials (parts [B*T][num_parts]) into logprob f32 [B, T], score f32
+// [B] and argmax int32 [B, T] (each may be nullptr), masked after the first eos among tokens[b, 1..T]
+struct LsePartial;
+int score_combine(cudaStream_t st, const LsePartial* parts, int num_parts, const int64_t* tokens, int ld_tok, int B,
+                  int T, int eos, int pad, float* logprob, float* score, int32_t* argmax);
 int pack_tokens(cudaStream_t st, const int64_t* tokens, int rows, int ld_tok, int sos, int eos, int pad, int32_t* lengths,
                 int32_t* packed);
 int init_decode(cudaStream_t st, DecodeState* state, int64_t* tokens, int ld_tok, int rows, int sos, int pad,

@@ -10,6 +10,8 @@ non-eos tokens (im2latex.py:33-39,50,55).  ``predict_batch`` is the tensor-batch
 
 ``beam_size > 1`` decodes with beam search instead (the reference app's ``DEFAULT_BEAM_SIZE``), and
 ``predict_nbest`` returns every image's ranked alternatives, each with the same confidence bookkeeping.
+``score_formulas`` goes the other way: it scores formulas the caller already has (a user's correction, candidates
+from elsewhere) against their images with one teacher-forced ``model.score`` call.
 """
 from __future__ import annotations
 
@@ -89,6 +91,40 @@ def predict_nbest(model, image_tensors: torch.Tensor, vocab: Dict[str, int], idx
     toks, lps, scs = tokens[:, :, 1:].cpu().tolist(), logp.cpu().tolist(), scores.cpu().tolist()
     eos = vocab[config.eos_token]
     return [rank_hypotheses(t, l, s, eos, idx2char) for t, l, s in zip(toks, lps, scs)]
+
+
+def formulas_to_ids(formulas: List[str], vocab: Dict[str, int], max_seq_len: int) -> torch.Tensor:
+    """Formulas in token form (vocabulary tokens separated by spaces, what ``inference.predict`` returns) ->
+    int64 ``[N, 1+T]``: sos, the token ids, eos, then pad up to the longest row (T = longest formula + 1).  An unknown
+    token or a formula longer than ``max_seq_len - 1`` tokens raises ValueError."""
+    sos, eos, pad = vocab[config.sos_token], vocab[config.eos_token], vocab[config.pad_token]
+    rows = []
+    for f in formulas:
+        toks = f.split()
+        unknown = [t for t in toks if t not in vocab]
+        if unknown:
+            raise ValueError(f"token {unknown[0]!r} of formula {f!r} is not in the vocabulary")
+        if len(toks) > max_seq_len - 1:
+            raise ValueError(f"formula of {len(toks)} tokens exceeds max_seq_len - 1 = {max_seq_len - 1}")
+        rows.append([sos] + [vocab[t] for t in toks] + [eos])
+    width = max(len(r) for r in rows)
+    return torch.tensor([r + [pad] * (width - len(r)) for r in rows], dtype=torch.int64)
+
+
+def score_formulas(model, image_tensors: torch.Tensor, formulas: List[str], vocab: Dict[str, int],
+                   idx2char: Dict[int, str], device: str = "cuda") -> List[Tuple[float, float]]:
+    """Score formula ``i`` (token form) against image ``i`` -> ``[(confidence, score), ...]``.  ``score`` is the
+    summed log-probability of the formula's tokens and its eos; ``confidence`` is ``predict``'s bookkeeping of the same
+    per-token log-probabilities, so for ``predict``'s own output it equals ``predict``'s confidence."""
+    if len(formulas) != image_tensors.shape[0]:
+        raise ValueError(f"{len(formulas)} formulas for {image_tensors.shape[0]} images")
+    model = model.to(device)
+    model.eval()
+    ids = formulas_to_ids(formulas, vocab, model.max_seq_len)
+    logp, scores = model.score(image_tensors, tokens=ids)
+    eos = vocab[config.eos_token]
+    toks, lps, scs = ids[:, 1:].tolist(), logp.cpu().tolist(), scores.cpu().tolist()
+    return [(_finish(t, l, eos, idx2char)[1], s) for t, l, s in zip(toks, lps, scs)]
 
 
 def predict_batch(model, image_tensors: torch.Tensor, vocab: Dict[str, int], idx2char: Dict[int, str],

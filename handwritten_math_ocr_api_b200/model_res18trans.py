@@ -90,3 +90,10 @@ class FormulaRecognitionModel(_Base):
             self.set_pos_table(pos_table)
         return super().generate_nbest(images, encoder_out=encoder_out, beam_size=beam_size, n_best=n_best,
                                       max_len=max_len)
+
+    @torch.no_grad()
+    def score(self, images=None, *, encoder_out=None, tokens, return_argmax: bool = False,
+              pos_table: Optional[torch.Tensor] = None):
+        if encoder_out is None:
+            self.set_pos_table(pos_table)
+        return super().score(images, encoder_out=encoder_out, tokens=tokens, return_argmax=return_argmax)

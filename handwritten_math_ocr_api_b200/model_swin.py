@@ -13,6 +13,7 @@ plus the one new entry point the engine exists for:
 
     tokens, steps, logprobs = model.generate(images, max_len=150, beam_size=1)
     tokens, scores, logprobs, steps = model.generate_nbest(images, beam_size=3)     # ranked beam hypotheses
+    logprobs, scores = model.score(images, tokens=tokens)                            # teacher-forced scoring
 
 Every tensor stays a torch CUDA tensor; torch is only the allocator / stream provider.  There is
 no CPU path: ``.to('cpu')`` raises, and a missing ``libhmocr.so`` raises at construction.
@@ -149,7 +150,7 @@ class FormulaRecognitionModel:
         self._n_params = 0
         # scratch memory is a torch tensor handed to the engine (SURVEY.md 8b "Ownership"): see _reserve
         self._workspace: Optional[torch.Tensor] = None
-        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0)}
+        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0), "score": (0, 0)}
         self.encoder = EncoderSwin(self)
         self.decoder = DecoderTransformer(self)
         self.training = False
@@ -275,6 +276,9 @@ class FormulaRecognitionModel:
             elif kind == "nbest":
                 b, t, k = self._reserved["nbest"]
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, -k, C.byref(n)), "hmocr_workspace_bytes")
+            elif kind == "score":
+                b, t = self._reserved["score"]
+                _lib.check(lib.hmocr_score_workspace_bytes(h, b, t, C.byref(n)), "hmocr_score_workspace_bytes")
             else:
                 b, t = self._reserved["tf"]
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, 0, C.byref(n)), "hmocr_workspace_bytes")
@@ -403,6 +407,40 @@ class FormulaRecognitionModel:
         return tokens[:, :, : t + 1], scores, logp[:, :, :t], t
 
     @torch.no_grad()
+    def score(self, images: Optional[torch.Tensor] = None, *, encoder_out: Optional[torch.Tensor] = None,
+              tokens: torch.Tensor, return_argmax: bool = False):
+        """Teacher-forced scoring of given sequences: how likely each formula is for its image.
+
+        ``tokens`` int64 ``[B, 1+T]`` in the layout ``generate`` returns (column 0 = sos, then the scored tokens; what
+        follows a row's first eos is ignored).  Returns ``(logprobs f32 [B, T], scores f32 [B])`` - the log-softmax of
+        each scored token up to and including the row's first eos (0 after it) and its fp32 sum in position order, the
+        definition of ``generate_nbest``'s scores - plus ``argmax`` int32 ``[B, T]`` (the model's own top token at each
+        position, lowest index on ties, pad after eos) when ``return_argmax``.  The logits are never materialised.
+        A bad shape raises ValueError, an id outside the vocabulary IndexError, T outside [1, max_seq_len]
+        RuntimeError."""
+        if (images is None) == (encoder_out is None):
+            raise ValueError("score: pass exactly one of images and encoder_out")
+        x = self._images(images) if encoder_out is None else self._memory(encoder_out)
+        B = x.shape[0]
+        tok = tokens.to(device=self.device, dtype=torch.int64).contiguous()
+        if tok.dim() != 2 or tok.shape[0] != B or tok.shape[1] < 1:
+            raise ValueError(f"tokens must be [B,1+T] with B={B}, got {tuple(tok.shape)}")
+        if int(tok.min()) < 0 or int(tok.max()) >= self.vocab_size:
+            raise IndexError("index out of range in self")         # what nn.Embedding raises
+        T = tok.shape[1] - 1
+        if 1 <= T <= self.max_seq_len:                              # otherwise the library call below names the problem
+            self._reserve("score", B, T)
+        logp = torch.empty(B, T, dtype=torch.float32, device=self.device)
+        scores = torch.empty(B, dtype=torch.float32, device=self.device)
+        argmax = torch.empty(B, T, dtype=torch.int32, device=self.device) if return_argmax else None
+        with torch.cuda.device(self.device):
+            _lib.check(self._eng.lib.hmocr_score(self._handle(), _ptr(x), int(encoder_out is not None), B, T, _ptr(tok),
+                                                 _ptr(logp), _ptr(scores), _ptr(argmax), _stream()), "hmocr_score")
+        if return_argmax:
+            return logp, scores, argmax
+        return logp, scores
+
+    @torch.no_grad()
     def pack_tokens(self, tokens: torch.Tensor):
         """Detokenise on the device (the per-id Python loop of /root/reference/src/inference.py:29-40): drops sos /
         pad ids, stops at the first eos.  ``tokens`` int64 ``[B, L]`` (CUDA) -> ``(packed int32 [B, L], lengths int32
@@ -421,7 +459,7 @@ class FormulaRecognitionModel:
         include/hmocr.h lists them)."""
         _lib.check(self._eng.lib.hmocr_set_option(self._eng.handle, name.encode(), int(value)), "hmocr_set_option")
         # options change which scratch buffers a call uses (step graph / tracing): plan again
-        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0)}
+        self._reserved = {"gen": (0, 0, 0), "nbest": (0, 0, 0), "tf": (0, 0), "score": (0, 0)}
 
     def last_decode_steps(self) -> int:
         """Decode steps the persistent kernel executed in the last ``generate`` call (after a stream synchronise): the

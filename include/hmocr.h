@@ -160,6 +160,27 @@ int hmocr_generate_nbest(hmocr_engine* e, const float* input_dev, int input_is_m
                          int n_best, int64_t* tokens_dev, float* logprob_dev, float* score_dev, int32_t* steps_dev,
                          void* stream);
 
+/* Teacher-forced scoring of given token sequences ("how likely is this formula for this image").
+ *   input_dev   images f32 [B,1,96,320] (input_is_memory == 0) or encoder output f32 [B,mem_tokens,d_model] (!= 0)
+ *   tokens_dev  int64 [B, 1+T], 1 <= T <= max_seq_len, ids in [0, vocab_size).  Column 0 is the first decoder input
+ *               (sos in normal use); columns 1..T are the scored tokens, the same layout hmocr_generate returns.
+ *   logprob_dev f32   [B, T]  log_softmax(logits at position t)[tokens[b, t+1]] up to and including the row's first
+ *                             eos among columns 1..T; 0 after it.  A row without eos is scored over all T.  (may be NULL)
+ *   score_dev   f32   [B]     fp32 sum of the row of logprob in position order, the same definition as
+ *                             hmocr_generate_nbest's score (may be NULL)
+ *   argmax_dev  int32 [B, T]  the model's most likely token at each position given the row's prefix, ties -> lowest
+ *                             index (the greedy rule); pad_id after the first eos (may be NULL)
+ * At least one output is non-NULL.  Ids after a row's first eos do not affect that row's outputs.
+ * The images form runs the encoder as hmocr_generate does (ResNet-18 variant: with the hmocr_set_pos_table table).
+ * The logits are never stored: fc_out runs with a log-sum-exp epilogue that keeps per-row partials of 128 columns,
+ * so a row's results do not depend on the batch it is scored in (DESIGN.md section 4.9). */
+int hmocr_score(hmocr_engine* e, const float* input_dev, int input_is_memory, int batch, int T,
+                const int64_t* tokens_dev, float* logprob_dev, float* score_dev, int32_t* argmax_dev, void* stream);
+
+/* Workspace of hmocr_score(batch, T), both input forms.  It shares the per-buffer maximum with
+ * hmocr_workspace_bytes, so the last answer of either function covers every shape asked of both. */
+int hmocr_score_workspace_bytes(hmocr_engine* e, int batch, int T, size_t* bytes);
+
 /* End-to-end form with HOST buffers (what `predict(images, model, vocab, idx2char, device)` does
  * around the model: images.to(device) ... ids back on the host): pinned or pageable host memory
  * in, host memory out, H2D and D2H inside, synchronises before returning. */
