@@ -1,5 +1,5 @@
-// Non-GEMM kernels of the Transformer decoder (sm_100a): token+position embedding, attention
-// (teacher-forced and single-step KV-cached), greedy selection with on-device bookkeeping.
+// Non-GEMM kernels of the Transformer decoder (sm_100a): token+position embedding, teacher-forced attention,
+// the on-device bookkeeping before and after a greedy decode, and the merge of the scoring partials.
 // Follows /root/reference/src/model_swin.py:72-88 and torch.nn.TransformerDecoderLayer
 // (post-LN; MultiheadAttention: 8 heads x 32, scores scaled by 1/sqrt(32), causal -inf mask).
 #include "gemm.cuh"
@@ -110,14 +110,13 @@ __global__ void __launch_bounds__(256) prefill_self_kernel(const h16* __restrict
 
 __global__ void __launch_bounds__(256) cross_kernel(const h16* __restrict__ q16,
                                                     const h16* __restrict__ memkv, int ld_mem, int koff,
-                                                    int voff, const int* __restrict__ mem_row, int rows, int T, int S,
-                                                    int nhead, h16* __restrict__ ctx) {
+                                                    int voff, int rows, int T, int S, int nhead, h16* __restrict__ ctx) {
   const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (w >= rows * nhead) return;
   const int lane = threadIdx.x & 31;
   const int h = w % nhead, r = w / nhead;       // r = b*T + t
   const int d = nhead * HD;
-  const int img = (mem_row != nullptr) ? mem_row[r] : (r / T);
+  const int img = r / T;
   float q[HD];
   load_row32(q16 + (size_t)r * d + h * HD, q);
 #pragma unroll
@@ -128,99 +127,6 @@ __global__ void __launch_bounds__(256) cross_kernel(const h16* __restrict__ q16,
       q, S, [&](int j) { return kb + (size_t)j * ld_mem; }, [&](int j) { return vb + (size_t)j * ld_mem; }, lane);
   ctx[(size_t)r * d + h * HD + lane] = to_h16(o);
 }
-
-// ---- single decode step --------------------------------------------------------------------------
-// cache layout: [row][head][tmax][32] fp16 (one layer); the new K/V row is written first, then the
-// whole warp reads positions 0..t (same-warp global store -> __syncwarp -> load is ordered).
-__global__ void __launch_bounds__(256) self_step_kernel(const DecodeState* __restrict__ state,
-                                                        const h16* __restrict__ qkv,
-                                                        h16* kcache, h16* vcache, int rows,
-                                                        int nhead, int tmax, h16* __restrict__ ctx) {
-  const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (w >= rows * nhead) return;
-  const int lane = threadIdx.x & 31;
-  const int h = w % nhead, r = w / nhead;
-  const int d = nhead * HD, pitch = 3 * d;
-  const int t = state->step;
-  const h16* row = qkv + (size_t)r * pitch + h * HD;
-  h16* kb = kcache + ((size_t)r * nhead + h) * tmax * HD;
-  h16* vb = vcache + ((size_t)r * nhead + h) * tmax * HD;
-  kb[(size_t)t * HD + lane] = row[d + lane];
-  vb[(size_t)t * HD + lane] = row[2 * d + lane];
-  __syncwarp();
-  float q[HD];
-  load_row32(row, q);
-#pragma unroll
-  for (int i = 0; i < HD; ++i) q[i] *= ATT_SCALE;
-  const float o = warp_attend(
-      q, t + 1, [&](int j) { return (const h16*)(kb + (size_t)j * HD); },
-      [&](int j) { return (const h16*)(vb + (size_t)j * HD); }, lane);
-  ctx[(size_t)r * d + h * HD + lane] = to_h16(o);
-}
-
-// ---- greedy selection ----------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) greedy_select_kernel(DecodeState* state, const float* __restrict__ logits,
-                                                            int ld, int n_valid, int64_t* __restrict__ tokens,
-                                                            int ld_tok, float* __restrict__ logprob, int max_len,
-                                                            int eos, uint8_t* __restrict__ finished,
-                                                            const float* __restrict__ emb,
-                                                            const float* __restrict__ pos, int d, int max_pos,
-                                                            float* __restrict__ x32, h16* __restrict__ x16,
-                                                            int rows) {
-  __shared__ float s_val[8];
-  __shared__ int s_idx[8];
-  __shared__ float s_sum[8];
-  const int r = blockIdx.x;
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int t = state->step;
-  const float* row = logits + (size_t)r * ld;
-  float best = -INFINITY;
-  int bi = 0x7fffffff;
-  for (int c = tid; c < n_valid; c += 256) {
-    const float v = row[c];
-    if (v > best) { best = v; bi = c; }       // strided scan keeps the lowest index per thread
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
-  }
-  if (lane == 0) { s_val[wid] = best; s_idx[wid] = bi; }
-  __syncthreads();
-  best = s_val[0]; bi = s_idx[0];
-#pragma unroll
-  for (int i = 1; i < 8; ++i)
-    if (s_val[i] > best || (s_val[i] == best && s_idx[i] < bi)) { best = s_val[i]; bi = s_idx[i]; }
-  float sum = 0.f;
-  for (int c = tid; c < n_valid; c += 256) sum += __expf(row[c] - best);
-  sum = warp_sum(sum);
-  if (lane == 0) s_sum[wid] = sum;
-  __syncthreads();
-  if (tid == 0) {
-    float tot = 0.f;
-    for (int i = 0; i < 8; ++i) tot += s_sum[i];
-    tokens[(size_t)r * ld_tok + t + 1] = bi;
-    if (logprob != nullptr) logprob[(size_t)r * max_len + t] = -logf(tot);   // log_softmax of the argmax
-    if (bi == eos && !finished[r]) {
-      finished[r] = 1;
-      const int c = atomicAdd(&state->finished_count, 1) + 1;
-      if (c == rows) state->steps_executed = t + 1;      // src/inference.py:23-25
-    }
-  }
-  // embedding of the chosen token at position t+1 for the next step
-  if (t + 1 < max_pos) {
-    for (int c = tid * 4; c < d; c += 1024) {
-      const float4 e = *reinterpret_cast<const float4*>(emb + (size_t)bi * d + c);
-      const float4 p = *reinterpret_cast<const float4*>(pos + (size_t)(t + 1) * d + c);
-      const float4 y = make_float4(e.x + p.x, e.y + p.y, e.z + p.z, e.w + p.w);
-      *reinterpret_cast<float4*>(x32 + (size_t)r * d + c) = y;
-      *reinterpret_cast<uint2*>(x16 + (size_t)r * d + c) = make_uint2(pack16(y.x, y.y), pack16(y.z, y.w));
-    }
-  }
-}
-
-__global__ void advance_step_kernel(DecodeState* state) { state->step += 1; }
 
 __global__ void init_decode_kernel(DecodeState* state, int64_t* tokens, int ld_tok, int rows, int sos, int pad,
                                    uint8_t* finished, float* logprob, int max_len) {
@@ -395,39 +301,7 @@ int mha_prefill_self(cudaStream_t st, const h16* qkv16, int B, int T, int nhead,
 int mha_prefill_cross(cudaStream_t st, const h16* q16, const h16* memkv, int ld_mem, int koff,
                       int voff, int B, int T, int S, int nhead, h16* ctx16) {
   HM_CHECK(S <= 32 * MAXK, "attention: S=%d exceeds %d", S, 32 * MAXK);
-  cross_kernel<<<ceil_div(B * T * nhead, 8), 256, 0, st>>>(q16, memkv, ld_mem, koff, voff, nullptr, B * T, T, S, nhead,
-                                                          ctx16);
-  HM_LAUNCHED();
-  return 0;
-}
-
-int self_attn_step(cudaStream_t st, const DecodeState* state, const h16* qkv16, h16* kcache,
-                   h16* vcache, int rows, int nhead, int tmax, h16* ctx16) {
-  HM_CHECK(tmax <= 32 * MAXK, "attention: max_len=%d exceeds %d", tmax, 32 * MAXK);
-  self_step_kernel<<<ceil_div(rows * nhead, 8), 256, 0, st>>>(state, qkv16, kcache, vcache, rows, nhead, tmax, ctx16);
-  HM_LAUNCHED();
-  return 0;
-}
-
-int cross_attn_step(cudaStream_t st, const h16* q16, const h16* memkv, int ld_mem, int koff,
-                    int voff, const int* mem_row, int rows, int S, int nhead, h16* ctx16) {
-  cross_kernel<<<ceil_div(rows * nhead, 8), 256, 0, st>>>(q16, memkv, ld_mem, koff, voff, mem_row, rows, 1, S, nhead,
-                                                         ctx16);
-  HM_LAUNCHED();
-  return 0;
-}
-
-int greedy_select(cudaStream_t st, DecodeState* state, const float* logits, int ld, int n_valid, int rows,
-                  int64_t* tokens, int ld_tok, float* logprob, int max_len, int eos, uint8_t* finished,
-                  const float* emb, const float* pos, int d, int max_pos, float* x32, h16* x16) {
-  greedy_select_kernel<<<rows, 256, 0, st>>>(state, logits, ld, n_valid, tokens, ld_tok, logprob, max_len, eos,
-                                             finished, emb, pos, d, max_pos, x32, x16, rows);
-  HM_LAUNCHED();
-  return 0;
-}
-
-int advance_step(cudaStream_t st, DecodeState* state) {
-  advance_step_kernel<<<1, 1, 0, st>>>(state);
+  cross_kernel<<<ceil_div(B * T * nhead, 8), 256, 0, st>>>(q16, memkv, ld_mem, koff, voff, B * T, T, S, nhead, ctx16);
   HM_LAUNCHED();
   return 0;
 }

@@ -40,7 +40,6 @@ constexpr int RES18_C[4] = {64, 128, 256, 512};
 constexpr int RES18_STRIDE[4] = {1, 2, 2, 2};
 constexpr int DEPTHS[4] = {2, 2, 6, 2};
 constexpr int HEADS[4] = {3, 6, 12, 24};
-constexpr int STEP_CHUNK = 8;     // decode steps between early-exit polls
 
 struct HostTensor {
   std::vector<float> f;
@@ -101,7 +100,6 @@ struct hmocr_engine {
   uint8_t* dp_wstream = nullptr;
   float* dp_lnparams = nullptr;
   int dp_fc_tiles = 0, dp_chunks_per_step = 0;
-  int decode_impl = 0;                // 0 = persistent cluster kernel, 1 = per-kernel step graph
   int steps_per_launch = 0;           // 0 = automatic (see generate_persistent)
   int trace_step = -1;                // >= 0: record phase-boundary clocks of that decode step
   int conv_impl = 0;                  // ResNet trunk: 0 = implicit GEMM (TMA patches), 1 = explicit im2col + GEMM
@@ -122,8 +120,6 @@ struct hmocr_engine {
   std::map<std::string, size_t> planned;   // per-buffer maximum over every hmocr_workspace_bytes call: placements use it,
                                            // so a small call followed by a large one never places a buffer twice
 
-  struct StepGraph { cudaGraphExec_t exec = nullptr; uint64_t epoch = 0; };
-  std::map<long long, StepGraph> graphs;   // key: rows
   // small batches: the ~95 encoder kernels are launch-bound, so generate() replays them as one captured graph
   struct EncGraph { cudaGraphExec_t exec = nullptr; uint64_t epoch = 0; bool warm = false; long launches = 0; };
   std::map<int, EncGraph> enc_graphs;      // key: batch
@@ -518,10 +514,9 @@ int project_memory(hmocr_engine* e, const h16* enc16, int B, h16* memkv, cudaStr
 struct DecBufs {
   float* x32;
   h16 *x16, *qkv, *q, *ctx, *hid;
-  float* logits;
 };
 
-// the activations of the layer stack; logits stays nullptr (hmocr_score keeps no logits)
+// the activations of the layer stack
 int dec_layer_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
   const int d = e->cfg.d_model, ff = e->cfg.dim_feedforward;
   std::string t(tag);
@@ -531,42 +526,6 @@ int dec_layer_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
   HM_TRY(ws_get(e, (t + ".q").c_str(), rows * d, &b->q));
   HM_TRY(ws_get(e, (t + ".ctx").c_str(), rows * d, &b->ctx));
   HM_TRY(ws_get(e, (t + ".hid").c_str(), rows * ff, &b->hid));
-  b->logits = nullptr;
-  return 0;
-}
-
-// the layer-stack activations plus the rows x vpad fp32 logits
-int dec_bufs(hmocr_engine* e, const char* tag, size_t rows, DecBufs* b) {
-  HM_TRY(dec_layer_bufs(e, tag, rows, b));
-  return ws_get(e, (std::string(tag) + ".logits").c_str(), rows * e->vpad, &b->logits);
-}
-
-// everything of one decoder layer after the self-attention context is in b.ctx
-int layer_tail(hmocr_engine* e, const DecLayer& L, int l, const DecBufs& b, int rows, const h16* memkv,
-               const int* mem_row, int T, cudaStream_t st) {
-  const int d = e->cfg.d_model, ff = e->cfg.dim_feedforward, nh = e->cfg.nhead;
-  GemmEpilogue e1;                       // x = LN1(x + out_proj(ctx))
-  e1.residual = b.x32; e1.ldr = d; e1.out_f32 = b.x32; e1.ld32 = d; e1.out_f16 = b.x16; e1.ld16 = d;
-  e1.ln_gamma = L.n1.g; e1.ln_beta = L.n1.b;
-  HM_TRY(run_lin(st, b.ctx, d, rows, L.sa_out, e1));
-  GemmEpilogue eq;
-  eq.out_f16 = b.q; eq.ld16 = d;
-  HM_TRY(run_lin(st, b.x16, d, rows, L.ca_q, eq));
-  if (T > 0)
-    HM_TRY(mha_prefill_cross(st, b.q, memkv, e->ca_kv.n, l * 2 * d, l * 2 * d + d, rows / T, T, e->mem_len, nh, b.ctx));
-  else
-    HM_TRY(cross_attn_step(st, b.q, memkv, e->ca_kv.n, l * 2 * d, l * 2 * d + d, mem_row, rows, e->mem_len, nh, b.ctx));
-  GemmEpilogue e2;                       // x = LN2(x + out_proj(ctx))
-  e2.residual = b.x32; e2.ldr = d; e2.out_f32 = b.x32; e2.ld32 = d; e2.out_f16 = b.x16; e2.ld16 = d;
-  e2.ln_gamma = L.n2.g; e2.ln_beta = L.n2.b;
-  HM_TRY(run_lin(st, b.ctx, d, rows, L.ca_out, e2));
-  GemmEpilogue ef;
-  ef.act = 2; ef.out_f16 = b.hid; ef.ld16 = ff;
-  HM_TRY(run_lin(st, b.x16, d, rows, L.l1, ef));
-  GemmEpilogue e3;                       // x = LN3(x + linear2(relu(linear1 x)))
-  e3.residual = b.x32; e3.ldr = d; e3.out_f32 = b.x32; e3.ld32 = d; e3.out_f16 = b.x16; e3.ld16 = d;
-  e3.ln_gamma = L.n3.g; e3.ln_beta = L.n3.b;
-  HM_TRY(run_lin(st, b.hid, ff, rows, L.l2, e3));
   return 0;
 }
 
@@ -578,7 +537,7 @@ int layer_tail(hmocr_engine* e, const DecLayer& L, int l, const DecBufs& b, int 
 // caller's fp32 encoder output and is converted into enc16 first; enc32 == nullptr: enc16 already holds it.
 int decoder_layers(hmocr_engine* e, const float* enc32, h16* enc16, h16* memkv, const int64_t* tok, int ld_tok, int B,
                    int T, const DecBufs& b, cudaStream_t st) {
-  const int d = e->cfg.d_model, nh = e->cfg.nhead;
+  const int d = e->cfg.d_model, ff = e->cfg.dim_feedforward, nh = e->cfg.nhead;
   const int rows = B * T;
   if (enc32 != nullptr) HM_TRY(f32_to_f16(st, enc32, (size_t)B * e->mem_len * d, enc16));
   HM_TRY(project_memory(e, enc16, B, memkv, st));
@@ -589,11 +548,30 @@ int decoder_layers(hmocr_engine* e, const float* enc32, h16* enc16, h16* memkv, 
     ei.out_f16 = b.qkv; ei.ld16 = 3 * d;
     HM_TRY(run_lin(st, b.x16, d, rows, L.sa_in, ei));
     HM_TRY(mha_prefill_self(st, b.qkv, B, T, nh, b.ctx));
-    HM_TRY(layer_tail(e, L, l, b, rows, memkv, nullptr, T, st));
+    GemmEpilogue e1;                     // x = LN1(x + out_proj(ctx))
+    e1.residual = b.x32; e1.ldr = d; e1.out_f32 = b.x32; e1.ld32 = d; e1.out_f16 = b.x16; e1.ld16 = d;
+    e1.ln_gamma = L.n1.g; e1.ln_beta = L.n1.b;
+    HM_TRY(run_lin(st, b.ctx, d, rows, L.sa_out, e1));
+    GemmEpilogue eq;
+    eq.out_f16 = b.q; eq.ld16 = d;
+    HM_TRY(run_lin(st, b.x16, d, rows, L.ca_q, eq));
+    HM_TRY(mha_prefill_cross(st, b.q, memkv, e->ca_kv.n, l * 2 * d, l * 2 * d + d, B, T, e->mem_len, nh, b.ctx));
+    GemmEpilogue e2;                     // x = LN2(x + out_proj(ctx))
+    e2.residual = b.x32; e2.ldr = d; e2.out_f32 = b.x32; e2.ld32 = d; e2.out_f16 = b.x16; e2.ld16 = d;
+    e2.ln_gamma = L.n2.g; e2.ln_beta = L.n2.b;
+    HM_TRY(run_lin(st, b.ctx, d, rows, L.ca_out, e2));
+    GemmEpilogue ef;
+    ef.act = 2; ef.out_f16 = b.hid; ef.ld16 = ff;
+    HM_TRY(run_lin(st, b.x16, d, rows, L.l1, ef));
+    GemmEpilogue e3;                     // x = LN3(x + linear2(relu(linear1 x)))
+    e3.residual = b.x32; e3.ldr = d; e3.out_f32 = b.x32; e3.ld32 = d; e3.out_f16 = b.x16; e3.ld16 = d;
+    e3.ln_gamma = L.n3.g; e3.ln_beta = L.n3.b;
+    HM_TRY(run_lin(st, b.hid, ff, rows, L.l2, e3));
   }
   return 0;
 }
 
+// the layer stack, then fc_out into a rows x vpad fp32 buffer and the first vocab_size columns out
 int decoder_forward_impl(hmocr_engine* e, const float* enc32, const int64_t* tgt, int B, int T, float* logits,
                          cudaStream_t st) {
   const int d = e->cfg.d_model;
@@ -602,135 +580,17 @@ int decoder_forward_impl(hmocr_engine* e, const float* enc32, const int64_t* tgt
   HM_TRY(ws_get(e, "tf.enc16", (size_t)B * e->mem_len * d, &enc16));
   HM_TRY(ws_get(e, "tf.memkv", (size_t)B * e->mem_len * e->ca_kv.n, &memkv));
   DecBufs b;
-  HM_TRY(dec_bufs(e, "tf", rows, &b));
+  float* logits32;
+  HM_TRY(dec_layer_bufs(e, "tf", rows, &b));
+  HM_TRY(ws_get(e, "tf.logits", (size_t)rows * e->vpad, &logits32));
   if (e->planning) return 0;
   HM_TRY(decoder_layers(e, enc32, enc16, memkv, tgt, T, B, T, b, st));
   GemmEpilogue eo;
-  eo.out_f32 = b.logits; eo.ld32 = e->vpad;
+  eo.out_f32 = logits32; eo.ld32 = e->vpad;
   HM_TRY(run_lin(st, b.x16, d, rows, e->fc, eo));
-  HM_TRY(copy_logits(st, b.logits, e->vpad, rows, e->cfg.vocab_size, logits));
+  HM_TRY(copy_logits(st, logits32, e->vpad, rows, e->cfg.vocab_size, logits));
   return 0;
 }
-
-// ------------------------------------------------------------------------------------------------
-// greedy generate              /root/reference/src/inference.py:15-25 with a KV cache
-// ------------------------------------------------------------------------------------------------
-struct GenBufs {
-  DecBufs b;
-  h16 *kcache, *vcache;   // [L][rows][nhead][tmax][32]
-  DecodeState* state;
-  uint8_t* finished;
-  int tmax;
-};
-
-int enqueue_step(hmocr_engine* e, const GenBufs& g, int rows, const h16* memkv, int64_t* tokens,
-                 float* logprob, int max_len, cudaStream_t st) {
-  const int d = e->cfg.d_model, nh = e->cfg.nhead;
-  const size_t layer_stride = (size_t)rows * nh * g.tmax * 32;
-  for (int l = 0; l < e->cfg.num_layers; ++l) {
-    const DecLayer& L = e->layers[l];
-    GemmEpilogue ei;
-    ei.out_f16 = g.b.qkv; ei.ld16 = 3 * d;
-    HM_TRY(run_lin(st, g.b.x16, d, rows, L.sa_in, ei));
-    HM_TRY(self_attn_step(st, g.state, g.b.qkv, g.kcache + l * layer_stride, g.vcache + l * layer_stride, rows, nh,
-                          g.tmax, g.b.ctx));
-    HM_TRY(layer_tail(e, L, l, g.b, rows, memkv, nullptr, 0, st));
-  }
-  GemmEpilogue eo;
-  eo.out_f32 = g.b.logits; eo.ld32 = e->vpad;
-  HM_TRY(run_lin(st, g.b.x16, d, rows, e->fc, eo));
-  HM_TRY(greedy_select(st, g.state, g.b.logits, e->vpad, e->cfg.vocab_size, rows, tokens, max_len + 1, logprob,
-                       max_len, e->cfg.eos_id, g.finished, e->emb, e->pos, d, e->cfg.max_seq_len, g.b.x32, g.b.x16));
-  HM_TRY(advance_step(st, g.state));
-  return 0;
-}
-
-int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam, int64_t* tokens,
-                        float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best);
-
-// n_best == 0: the hmocr_generate contract (best hypothesis only; logprob zero-filled in beam mode).
-// n_best >= 1: the hmocr_generate_nbest contract (beam machinery always; tokens / logprob / score hold n_best
-// hypotheses per image).  The step-graph decode is greedy only, so n-best always takes the persistent kernel.
-int generate_from_memory_impl(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam,
-                              int64_t* tokens, float* logprob, int32_t* steps, float* score, cudaStream_t st,
-                              int n_best = 0) {
-  HM_CHECK(max_len >= 1 && max_len <= e->cfg.max_seq_len,
-           "max_len=%d outside [1, %d] (size of pos_encoder, src/model_swin.py:54)", max_len, e->cfg.max_seq_len);
-  HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
-  // The beam kernel merges per-hypothesis top-`beam` token lists; with fewer tokens than hypotheses a list has empty
-  // slots, and the candidate built from one (hyp * vocab + 0x7fffffff) overflows into a negative parent index.
-  HM_CHECK(beam <= e->cfg.vocab_size, "beam=%d exceeds vocab_size=%d", beam, e->cfg.vocab_size);
-  if (e->decode_impl == 0 || n_best > 0)
-    return generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
-  HM_CHECK(beam == 1, "the step-graph decode (decode_impl=1) is greedy only; beam=%d needs decode_impl=0", beam);
-  const int d = e->cfg.d_model, nh = e->cfg.nhead, L = e->cfg.num_layers;
-  const int rows = B;
-  h16* memkv;
-  HM_TRY(ws_get(e, "gen.memkv", (size_t)B * e->mem_len * e->ca_kv.n, &memkv));
-  GenBufs g;
-  g.tmax = e->cfg.max_seq_len;
-  HM_TRY(dec_bufs(e, "gen", rows, &g.b));
-  const size_t cache_elems = (size_t)L * rows * nh * g.tmax * 32;
-  HM_TRY(ws_get(e, "gen.kcache", cache_elems, &g.kcache));
-  HM_TRY(ws_get(e, "gen.vcache", cache_elems, &g.vcache));
-  HM_TRY(ws_get(e, "gen.state", 1, &g.state));
-  HM_TRY(ws_get(e, "gen.finished", rows, &g.finished));
-  // per-call output pointers are baked into the step graph: stage them in engine-owned buffers
-  int64_t* tok_ws;
-  float* lp_ws;
-  HM_TRY(ws_get(e, "gen.tokens", (size_t)rows * (g.tmax + 1), &tok_ws));
-  HM_TRY(ws_get(e, "gen.logprob", (size_t)rows * g.tmax, &lp_ws));
-  if (e->planning) return 0;
-
-  HM_TRY(project_memory(e, enc16, B, memkv, st));
-  HM_TRY(init_decode(st, g.state, tok_ws, max_len + 1, rows, e->cfg.sos_id, e->cfg.pad_id, g.finished, lp_ws, max_len));
-  HM_TRY(embed_tokens(st, tok_ws, max_len + 1, rows, 1, e->emb, e->pos, d, e->cfg.vocab_size, g.b.x32, g.b.x16));
-
-  // one decode step captured once per (rows, max_len) and replayed: the step index lives in HBM
-  const long long key = (long long)rows * 1024 + max_len;
-  hmocr_engine::StepGraph& sg = e->graphs[key];
-  if (sg.exec == nullptr || sg.epoch != e->ws_epoch) {
-    if (sg.exec != nullptr) { cudaGraphExecDestroy(sg.exec); sg.exec = nullptr; }
-    cudaGraph_t graph = nullptr;
-    HM_CUDA(cudaStreamBeginCapture(e->cap_stream, cudaStreamCaptureModeThreadLocal));
-    const long launches_before = g_launch_count;
-    int rc = enqueue_step(e, g, rows, memkv, tok_ws, lp_ws, max_len, e->cap_stream);
-    g_launch_count = launches_before;            // captured, not launched
-    cudaError_t ce = cudaStreamEndCapture(e->cap_stream, &graph);
-    if (rc != 0) { if (graph) cudaGraphDestroy(graph); return rc; }
-    HM_CUDA(ce);
-    ce = cudaGraphInstantiate(&sg.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    HM_CUDA(ce);
-    sg.epoch = e->ws_epoch;
-  }
-  size_t nodes_per_step = 8 * (size_t)L + 3;
-  int launched_steps = 0, poll_idx = 0;
-  bool done = false;
-  for (int s0 = 0; s0 < max_len && !done; s0 += STEP_CHUNK, ++poll_idx) {
-    const int n = (max_len - s0 < STEP_CHUNK) ? (max_len - s0) : STEP_CHUNK;
-    for (int i = 0; i < n; ++i) {
-      HM_CUDA(cudaGraphLaunch(sg.exec, st));
-      g_launch_count += (long)nodes_per_step;
-    }
-    launched_steps += n;
-    const int slot = poll_idx & 1;
-    HM_CUDA(cudaMemcpyAsync(&e->pinned_state[slot], g.state, sizeof(DecodeState), cudaMemcpyDeviceToHost, st));
-    HM_CUDA(cudaEventRecord(e->poll_ev[slot], st));
-    if (poll_idx >= 1) {                         // look at the chunk before: the GPU never idles
-      const int prev = (poll_idx - 1) & 1;
-      HM_CUDA(cudaEventSynchronize(e->poll_ev[prev]));
-      if (e->pinned_state[prev].steps_executed > 0) done = true;   // every row has emitted eos
-    }
-  }
-  (void)launched_steps;
-  HM_TRY(finalize_decode(st, g.state, tok_ws, max_len + 1, rows, max_len, e->cfg.pad_id, lp_ws, steps));
-  HM_CUDA(cudaMemcpyAsync(tokens, tok_ws, sizeof(int64_t) * rows * (max_len + 1), cudaMemcpyDeviceToDevice, st));
-  if (logprob != nullptr)
-    HM_CUDA(cudaMemcpyAsync(logprob, lp_ws, sizeof(float) * rows * max_len, cudaMemcpyDeviceToDevice, st));
-  return 0;
-}
-
 
 // ------------------------------------------------------------------------------------------------
 // operand packing for decode_persistent.cu (host side, once at load)
@@ -818,11 +678,19 @@ int pack_decode_operands(hmocr_engine* e) {
 // the all-finished flag of the PREVIOUS launch (the GPU never idles).  beam == 1: greedy
 // (src/inference.py:15-25).  beam > 1 (or n_best > 0, at any beam): beam search as defined in
 // oracle/decode.py::beam_search - rows = images x beam hypotheses, two K/V cache sets, back-track at the end.
+// n_best == 0: the hmocr_generate contract (best hypothesis only; logprob zero-filled in beam mode).
+// n_best >= 1: the hmocr_generate_nbest contract (beam machinery always; tokens / logprob / score hold n_best
+// hypotheses per image).
 int generate_persistent(hmocr_engine* e, const h16* enc16, int B, int max_len, int beam, int64_t* tokens,
                         float* logprob, int32_t* steps, float* score, cudaStream_t st, int n_best) {
+  HM_CHECK(max_len >= 1 && max_len <= e->cfg.max_seq_len,
+           "max_len=%d outside [1, %d] (size of pos_encoder, src/model_swin.py:54)", max_len, e->cfg.max_seq_len);
+  HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
+  // The beam kernel merges per-hypothesis top-`beam` token lists; with fewer tokens than hypotheses a list has empty
+  // slots, and the candidate built from one (hyp * vocab + 0x7fffffff) overflows into a negative parent index.
+  HM_CHECK(beam <= e->cfg.vocab_size, "beam=%d exceeds vocab_size=%d", beam, e->cfg.vocab_size);
   const int nh = e->cfg.nhead, L = e->cfg.num_layers, rows = B * beam;
   const bool beam_mode = beam > 1 || n_best > 0;
-  HM_CHECK(beam >= 1 && beam <= DP_MAX_BEAM, "beam=%d outside [1, %d]", beam, DP_MAX_BEAM);
   float* memkv;                       // memory K/V of all layers, fp32 out of the GEMM, fp16 after the repack
   __half *memk, *memv, *kcache, *vcache;
   DecodeState* state;
@@ -990,7 +858,7 @@ int generate_impl(hmocr_engine* e, const float* images, int B, int max_len, int 
   HM_TRY(ws_get(e, "gen.enc16", (size_t)B * e->mem_len * e->cfg.d_model, &enc16));
   if (e->planning) {
     HM_TRY(encode_for_generate(e, images, B, enc32, enc16, st));
-    return generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
+    return generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best);
   }
   HM_CUDA(cudaEventRecord(e->ev[0], st));
   nvtx_push("hmocr.encode");
@@ -998,7 +866,7 @@ int generate_impl(hmocr_engine* e, const float* images, int B, int max_len, int 
   nvtx_pop();
   HM_TRY(rc_enc);
   HM_CUDA(cudaEventRecord(e->ev[1], st));
-  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
+  HM_TRY(generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
   HM_CUDA(cudaEventRecord(e->ev[2], st));
   e->timings_pending = true;
   return 0;
@@ -1012,7 +880,7 @@ int generate_from_enc32(hmocr_engine* e, const float* enc_out, int B, int max_le
   HM_TRY(f32_to_f16(st, enc_out, (size_t)B * e->mem_len * e->cfg.d_model, enc16));
   HM_CUDA(cudaEventRecord(e->ev[0], st));
   HM_CUDA(cudaEventRecord(e->ev[1], st));
-  HM_TRY(generate_from_memory_impl(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
+  HM_TRY(generate_persistent(e, enc16, B, max_len, beam, tokens, logprob, steps, score, st, n_best));
   HM_CUDA(cudaEventRecord(e->ev[2], st));
   e->timings_pending = true;
   return 0;
@@ -1160,8 +1028,6 @@ HM_API void hmocr_destroy(hmocr_engine* e) {
   if (e == nullptr) return;
   cudaSetDevice(e->device);
   cudaDeviceSynchronize();
-  for (auto& kv : e->graphs)
-    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
   for (auto& kv : e->enc_graphs)
     if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
   for (auto& kv : e->ws) {
@@ -1365,10 +1231,7 @@ HM_API int hmocr_decode_max_clusters(int* out) {
 HM_API int hmocr_set_option(hmocr_engine* e, const char* name, int value) {
   HM_CHECK(e != nullptr && name != nullptr, "hmocr_set_option: null argument");
   const std::string n(name);
-  if (n == "decode_impl") {
-    HM_CHECK(value == 0 || value == 1, "decode_impl must be 0 (persistent cluster kernel) or 1 (step graph)");
-    e->decode_impl = value;
-  } else if (n == "steps_per_launch") {
+  if (n == "steps_per_launch") {
     HM_CHECK(value >= 0 && value <= 256, "steps_per_launch must be in [0,256] (0 = automatic)");
     e->steps_per_launch = value;
   } else if (n == "trace_step") {

@@ -22,7 +22,7 @@ int swin_mlp(cudaStream_t st, const h16* xn, int M, int C, const h16* w1, const 
 
 // ---- decoder -------------------------------------------------------------------------------------
 struct DecodeState {      // device-resident control block of one generate call
-  int step;               // current decode step t (position of the token being fed)
+  int step;               // steps actually run, raised by atomicMax in the persistent kernel
   int finished_count;     // rows that have emitted eos at least once
   int steps_executed;     // ys.shape[1]-1 of the reference once every row has finished, else 0
   int last_eos;           // max over the finished rows (beam: clusters) of (step of the first eos) + 1.  Clusters of the
@@ -44,20 +44,6 @@ int mha_full_mma(cudaStream_t st, const h16* qkv, int B, int T, int nhead, h16* 
 int mha_prefill_cross(cudaStream_t st, const h16* q16, const h16* memkv, int ld_mem, int koff,
                       int voff, int B, int T, int S, int nhead, h16* ctx16);
 
-// one decode step, one warp per (row, head).  `mem_row` maps a decode row to its image (beam search:
-// several hypotheses share one image's memory K/V); nullptr = identity.
-int self_attn_step(cudaStream_t st, const DecodeState* state, const h16* qkv16, h16* kcache,
-                   h16* vcache, int rows, int nhead, int tmax, h16* ctx16);
-int cross_attn_step(cudaStream_t st, const h16* q16, const h16* memkv, int ld_mem, int koff,
-                    int voff, const int* mem_row, int rows, int S, int nhead, h16* ctx16);
-
-// greedy head: argmax (first max) + log-softmax of the winner over logits[rows, ld] (n_valid
-// columns), append to tokens[:, t+1], update finished bookkeeping, and embed the chosen token
-// for step t+1 (src/inference.py:20-24 + src/model_swin.py:73-75).
-int greedy_select(cudaStream_t st, DecodeState* state, const float* logits, int ld, int n_valid, int rows,
-                  int64_t* tokens, int ld_tok, float* logprob, int max_len, int eos, uint8_t* finished,
-                  const float* emb, const float* pos, int d, int max_pos, float* x32, h16* x16);
-int advance_step(cudaStream_t st, DecodeState* state);
 // teacher-forced scoring: merge the gemm_f16_lse partials (parts [B*T][num_parts]) into logprob f32 [B, T], score f32
 // [B] and argmax int32 [B, T] (each may be nullptr), masked after the first eos among tokens[b, 1..T]
 struct LsePartial;

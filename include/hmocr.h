@@ -68,8 +68,6 @@ int hmocr_load_weight(hmocr_engine* e, const char* key, const void* data_host, c
 int hmocr_finalize_weights(hmocr_engine* e);
 
 /* Engine options (all have working defaults):
- *   "decode_impl"       0 = persistent thread-block-cluster decode kernel (default)
- *                       1 = one captured CUDA graph of per-layer kernels per step (kept for A/B tests)
  *   "steps_per_launch"  decode steps per persistent-kernel launch; 0 (default) = automatic: one launch for the whole
  *                       decode when all clusters of the batch are co-resident (the kernel stops by itself once every
  *                       row has emitted eos), 16-step launches with a host poll in between for multi-wave batches

@@ -232,27 +232,6 @@ def test_incremental_decode_matches_teacher_forced(model, golden_src):
     assert (near < 1.5e-2).all()
 
 
-def test_persistent_kernel_agrees_with_step_graph(model, golden_src):
-    """Two independent implementations of the decode step (cluster kernel vs per-layer kernels)."""
-    feats = torch.from_numpy(golden_src["features"]).cuda()
-    a_tok, a_steps, a_lp = model.generate(encoder_out=feats, max_len=30, return_logprobs=True)
-    model.set_option("decode_impl", 1)
-    try:
-        b_tok, b_steps, b_lp = model.generate(encoder_out=feats, max_len=30, return_logprobs=True)
-    finally:
-        model.set_option("decode_impl", 0)
-    margin = golden_src["greedy_margin"]
-    for r in range(4):
-        d = (a_tok[r] != b_tok[r]).nonzero()
-        if d.numel():
-            c = int(d[0])
-            assert float(margin[r, c - 1]) < 2 * LOGIT_TOL      # only near-ties may differ
-            n = c - 1
-        else:
-            n = a_steps
-        assert (a_lp[r, :n] - b_lp[r, :n]).abs().max().item() < 1.5e-2
-
-
 @pytest.mark.parametrize("steps_per_launch", [1, 7, 64])
 def test_persistent_kernel_launch_chunking(model, golden_src, steps_per_launch):
     """Splitting the step range over several launches must not change a single token."""
@@ -264,6 +243,12 @@ def test_persistent_kernel_launch_chunking(model, golden_src, steps_per_launch):
     finally:
         model.set_option("steps_per_launch", 0)          # back to the automatic policy
     assert steps == ref_steps and torch.equal(tok, ref_tok)
+
+
+def test_removed_step_graph_switch_is_an_unknown_option(model):
+    """The persistent kernel is the only greedy decoder: the old step-graph switch is refused by name."""
+    with pytest.raises(RuntimeError, match="unknown option"):
+        model.set_option("decode_impl", 1)
 
 
 @pytest.mark.parametrize("B", [1, 15, 17, 33])
