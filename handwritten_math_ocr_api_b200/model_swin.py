@@ -265,25 +265,28 @@ class FormulaRecognitionModel:
         have = self._reserved[kind]
         if all(a >= b for a, b in zip(have, shape)):
             return
-        self._reserved[kind] = tuple(max(a, b) for a, b in zip(have, shape))
+        # recorded only once the engine has accepted the shape: a refused one (a ResNet-18 batch above 256) must not
+        # make every later plan of this kind include it
+        want = tuple(max(a, b) for a, b in zip(have, shape))
         lib, h = self._eng.lib, self._handle()
         n = C.c_size_t()
         with torch.cuda.device(self.device):
             # the engine keeps the per-buffer maximum over every shape asked so far: `n` covers all of them
             if kind == "gen":
-                b, t, k = self._reserved["gen"]
+                b, t, k = want
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, k, C.byref(n)), "hmocr_workspace_bytes")
             elif kind == "nbest":
-                b, t, k = self._reserved["nbest"]
+                b, t, k = want
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, -k, C.byref(n)), "hmocr_workspace_bytes")
             elif kind == "score":
-                b, t = self._reserved["score"]
+                b, t = want
                 _lib.check(lib.hmocr_score_workspace_bytes(h, b, t, C.byref(n)), "hmocr_score_workspace_bytes")
             else:
-                b, t = self._reserved["tf"]
+                b, t = want
                 _lib.check(lib.hmocr_workspace_bytes(h, b, t, 0, C.byref(n)), "hmocr_workspace_bytes")
             ws = torch.empty(n.value, dtype=torch.uint8, device=self.device)
             _lib.check(lib.hmocr_set_workspace(h, _ptr(ws), n.value, _stream()), "hmocr_set_workspace")
+        self._reserved[kind] = want
         self._workspace = ws                                     # the old tensor goes back to torch's allocator
 
     def workspace_bytes(self) -> int:
